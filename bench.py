@@ -30,8 +30,13 @@ clouds).  Prints ONE JSON line (rank 0).
   cpu_baseline  the same workload on the host cores (FPS: oracle port — the reference has no CPU
              FPS; ball query + group: the reference's own CPU functions when oracle/_ref travelled).
 
-Extra (not part of the driver contract): --report FILE writes per-kernel tables for all
-BASELINE.json configs; --fps-sweep / --bq-sweep time kernel variants.
+--dump-outputs DIR writes what the timed device-resident leg returned in its last step (rank 0):
+DIR/{fps_idx,new_xyz,idx,pts_cnt,grouped_xyz}.npy, float64 for the index tensors (exact) and float32
+for the coordinates, 22 MB at the default workload.  The inputs are seeded, so two builds run with
+the same arguments can be compared output for output.
+
+Extra: --report FILE writes per-kernel tables for all BASELINE.json configs; --fps-sweep /
+--bq-sweep time kernel variants.
 """
 from __future__ import annotations
 
@@ -48,6 +53,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 
 METRIC = "set-abstraction points/sec"
 UNIT = "points/s"
@@ -330,6 +336,14 @@ def child_json(argv, key, timeout=600.0):
 
 
 # ------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir: str, o: dict) -> None:
+    """The layer's outputs as a caller receives them: index tensors as float64 (exact), coordinates as float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, key in (("fps_idx", "fps_idx"), ("new_xyz", "new_xyz"), ("idx", "idx"), ("pts_cnt", "cnt"), ("grouped_xyz", "grouped")):
+        a = o[key].cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64 if a.dtype.kind == "i" else np.float32))
+
+
 def run_b200_arm(args, cfg):
     import ctypes
 
@@ -633,6 +647,8 @@ def run_b200_arm(args, cfg):
         elif configs_block is None:
             configs_block = {"error": "the configs block failed on another rank"}
 
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, fus)  # no later leg writes `fus`: it holds the last timed step's outputs
     if rank == 0:
         pt, pp, pc = ctypes.c_int(), ctypes.c_int(), ctypes.c_int()
         lib.pn2_fps_plan(b, n, ctypes.byref(pt), ctypes.byref(pp), ctypes.byref(pc))
@@ -721,6 +737,8 @@ def main():
     ap.add_argument("--in-flight", type=int, default=4, help="batches in flight in the secondary device-resident leg")
     ap.add_argument("--e2e-depth", type=int, default=3, help="batches in flight in the end-to-end leg")
     ap.add_argument("--report", type=str, default=None, help="write per-kernel tables for all BASELINE configs to this file")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="write the timed leg's outputs of its last step to DIR/<name>.npy")
     ap.add_argument("--fps-sweep", action="store_true")
     ap.add_argument("--bq-sweep", action="store_true")
     args = ap.parse_args()

@@ -53,7 +53,7 @@ def lib() -> ctypes.CDLL:
 
 
 def have_refcpu() -> bool:
-    return os.path.exists(os.path.join(HERE, "_ref", "libref_cpu.so")) or os.path.isdir("/root/reference")
+    return os.path.exists(os.path.join(HERE, "_ref", "libref_cpu.so"))
 
 
 def have_refcuda() -> bool:

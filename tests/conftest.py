@@ -1,3 +1,4 @@
+import hashlib
 import os
 import sys
 
@@ -37,6 +38,21 @@ def load_golden(name: str):
     if not os.path.exists(path):
         pytest.skip(f"golden fixture {name}.npz not generated yet (oracle/gen_golden.py)")
     return dict(np.load(path))
+
+
+def assert_golden_rows(got, g, case: str, output: str) -> None:
+    """``got`` equals the reference's output ``case/output`` stored by oracle/gen_golden.py
+    (ref_{cpu,cuda}_cases.npz) bit for bit: its stored rows first (a readable diff), then the whole
+    output through its shape and the sha256 of its bytes."""
+    if hasattr(got, "detach"):
+        got = got.detach().cpu().numpy()
+    got = np.ascontiguousarray(got)
+    key = f"{case}/{output}"
+    want = g[key]
+    assert got.dtype == want.dtype, (got.dtype, want.dtype)
+    np.testing.assert_array_equal(got.reshape(got.shape[0] * got.shape[1], -1)[g[f"{case}/pos"]], want)
+    assert got.shape == tuple(g[key + ".shape"]), (got.shape, tuple(g[key + ".shape"]))
+    assert hashlib.sha256(got.tobytes()).hexdigest() == str(g[key + ".sha256"]), f"{key}: differs outside the stored rows"
 
 
 def golden_names(prefix: str):

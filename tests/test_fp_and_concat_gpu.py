@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 import torch
 
+from conftest import assert_golden_rows, load_golden
 from oracle import oracle as O
 from pointnet2_b200 import _lib, tf_interpolate as TI, workloads as W
 from pointnet2_b200.pointnet_util import group_and_concat, pointnet_fp_module
@@ -79,8 +80,7 @@ def test_three_interpolate_grad_deterministic_matches_reference_order(dev, b, n,
     w = np.random.RandomState(213).random_sample((b, n, 3)).astype(np.float32)
     go = W.features(b, n, c, 214)
     want = O.oracle_three_interpolate_grad((b, m, c), idx, w, go)  # the C restatement adds in the reference's (j, t) order
-    if O.have_refcpu():
-        np.testing.assert_array_equal(O.refcpu_three_interpolate_grad((b, m, c), idx, w, go), want)
+    assert_golden_rows(want, load_golden("ref_cpu_cases"), f"three_interp_grad_det/{b}_{n}_{m}_{c}", "out")
     gp = torch.full((b, m, c), 7.0, dtype=torch.float32, device=dev)  # no zero-fill needed: overwritten
     wsb = int(lib.pn2_three_interpolate_grad_det_workspace_bytes(b, n, m))
     ws = torch.empty(wsb, dtype=torch.uint8, device=dev)

@@ -1,10 +1,12 @@
 """Parity at BASELINE.json's own sizes against the reference's own code (VERDICT r1, items 1):
-the reference CUDA kernels rebuilt for sm_100a and the reference CPU functions (oracle/_ref/, which
-travels to the GPU box).  Every index tensor bit-exact; three_interpolate bit-exact (contract 1e-5)."""
+the outputs of the reference CUDA kernels rebuilt for sm_100a and of the reference CPU functions on
+these tests' inputs (tests/golden/ref_cuda_cases.npz, a seeded sample of rows per case).  Every index
+tensor bit-exact; three_interpolate bit-exact (contract 1e-5)."""
 import numpy as np
 import pytest
 import torch
 
+from conftest import assert_golden_rows, load_golden
 from oracle import oracle as O
 from pointnet2_b200 import _lib, workloads as W
 from pointnet2_b200.tf_grouping import knn_point, query_ball_point
@@ -12,8 +14,6 @@ from pointnet2_b200.tf_interpolate import three_interpolate, three_nn, three_nn_
 from pointnet2_b200.tf_sampling import farthest_point_sample, farthest_point_sample_and_gather, gather_point
 
 pytestmark = pytest.mark.gpu
-needs_refcuda = pytest.mark.skipif(not O.have_refcuda(), reason="oracle/_ref CUDA libraries did not travel")
-needs_refcpu = pytest.mark.skipif(not O.have_refcpu(), reason="oracle/_ref CPU library did not travel")
 
 
 def T(a, dev):
@@ -21,19 +21,17 @@ def T(a, dev):
 
 
 # ---- cfg5: ball query at N = 65536 and 262144, M = N/4, S = 32, r = 0.1 (tf_grouping_g.cu:3-36) ------------
-@needs_refcuda
 @pytest.mark.parametrize("b,n", [(2, 65536), (1, 262144)])
 def test_cfg5_ball_query_matches_reference_kernel(dev, b, n):
     m = n // 4
     x = T(W.cloud_uniform(b, n, 100 + int(np.log2(n))), dev)
     _, nx = farthest_point_sample_and_gather(m, x)
     idx, cnt = query_ball_point(0.1, 32, x, nx)
-    ridx, rcnt = O.refcuda_query_ball_point(0.1, 32, x, nx)
-    assert torch.equal(cnt, rcnt)
-    assert torch.equal(idx, ridx)
+    g = load_golden("ref_cuda_cases")
+    assert_golden_rows(cnt, g, f"cfg5_bq/{b}_{n}", "cnt")
+    assert_golden_rows(idx, g, f"cfg5_bq/{b}_{n}", "idx")
 
 
-@needs_refcuda
 def test_cfg5_ball_query_sparse_radius_matches_reference_kernel(dev):
     """Same size with balls that do NOT fill up (r = 0.01: ~1 neighbour), so every query scans its
     whole neighbourhood and the padding path runs on every row."""
@@ -41,21 +39,22 @@ def test_cfg5_ball_query_sparse_radius_matches_reference_kernel(dev):
     x = T(W.cloud_uniform(b, n, 116), dev)
     nx = x[:, ::4].contiguous()
     idx, cnt = query_ball_point(0.01, 32, x, nx)
-    ridx, rcnt = O.refcuda_query_ball_point(0.01, 32, x, nx)
-    assert torch.equal(cnt, rcnt) and torch.equal(idx, ridx)
+    g = load_golden("ref_cuda_cases")
+    assert_golden_rows(cnt, g, "cfg5_bq_sparse", "cnt")
+    assert_golden_rows(idx, g, "cfg5_bq_sparse", "idx")
 
 
 # ---- cfg5: FPS at the largest sizes (tf_sampling_g.cu:105-170) ---------------------------------------------
-@needs_refcuda
 @pytest.mark.parametrize("gen,b,n,m", [("U", 1, 262144, 640), ("D", 2, 262144, 512), ("U", 2, 131073, 512), ("U", 8, 65536, 1024),
                                        ("D", 8, 16384, 2048)])
 def test_large_fps_matches_reference_kernel(dev, gen, b, n, m):
     x = T(W.DISTRIBUTIONS[gen](b, n, 118), dev)
+    g, case = load_golden("ref_cuda_cases"), f"fps_large/{gen}_{b}_{n}_{m}"
     idx = farthest_point_sample(m, x)
-    ref = O.refcuda_fps(m, x)
-    assert torch.equal(idx, ref)
+    assert_golden_rows(idx, g, case, "idx")
     fi, fx = farthest_point_sample_and_gather(m, x)
-    assert torch.equal(fi, ref) and torch.equal(fx, O.refcuda_gather_point(x, ref))
+    assert torch.equal(fi, idx)
+    assert_golden_rows(fx, g, case, "new_xyz")
 
 
 def test_eight_clouds_of_262144_points_run_as_co_resident_clusters(dev):
@@ -77,10 +76,10 @@ def test_eight_clouds_of_262144_points_run_as_co_resident_clusters(dev):
 
 
 # ---- cfg4: the whole FP stack at B = 16 (tf_interpolate.cpp:60-127) ------------------------------------------
-@needs_refcpu
 def test_cfg4_fp_stack_matches_reference_cpu_functions(dev):
     c4 = W.CFG4_SEMSEG
     b = c4["b"]
+    g = load_golden("ref_cuda_cases")
     xyz = W.cloud_duplicates(b, c4["n"], 100)
     x = T(xyz, dev)
     levels = {c4["n"]: x}
@@ -93,32 +92,20 @@ def test_cfg4_fp_stack_matches_reference_cpu_functions(dev):
         x1, x2 = levels[n], levels[m]
         p2 = W.features(b, m, c, 105)
         dist, idx = three_nn(x1, x2)
-        rd, ri = O.refcpu_three_nn(x1.cpu().numpy(), x2.cpu().numpy())
-        np.testing.assert_array_equal(idx.cpu().numpy(), ri)
-        np.testing.assert_array_equal(dist.cpu().numpy(), rd)
+        assert_golden_rows(idx, g, f"cfg4_fp/{n}_{m}", "idx")
+        assert_golden_rows(dist, g, f"cfg4_fp/{n}_{m}", "dist")
         d = torch.clamp(dist, min=1e-10)
         w = (1.0 / d) / (1.0 / d).sum(dim=2, keepdim=True)
         out = three_interpolate(T(p2, dev), idx, w)
-        ro = O.refcpu_three_interpolate(p2, ri, w.cpu().numpy())
-        assert np.abs(out.cpu().numpy() - ro).max() <= 1e-5
-        np.testing.assert_array_equal(out.cpu().numpy(), ro)  # in fact bit-exact
+        assert_golden_rows(out, g, f"cfg4_fp/{n}_{m}", "out")  # bit-exact (contract 1e-5)
         fused = three_nn_interpolate(x1, x2, T(p2, dev))
         assert float((fused - out).abs().max()) <= 1e-5
 
 
 # ---- n3: knn_point against the reference's composite (tf_grouping.py:48-73 + selection_sort_gpu) -------------
-def _knn_reference_composite(k, x1, x2):
-    """pairwise squared distances as the reference's graph computes them (tile, subtract, square,
-    reduce_sum over the 3 coordinates: each product rounded, summed left to right), then the rebuilt
-    selection_sort_gpu; the first k columns are knn_point's outputs."""
-    diff = x1.unsqueeze(1) - x2.unsqueeze(2)  # (b,m,n,3)
-    sq = diff * diff
-    dist = (sq[..., 0] + sq[..., 1]) + sq[..., 2]
-    outi, out = O.refcuda_selection_sort(k, dist.contiguous())
-    return out[:, :, :k].contiguous(), outi[:, :, :k].contiguous()
-
-
-@needs_refcuda
+# The reference composite: pairwise squared distances as the reference's graph computes them (tile, subtract,
+# square, reduce_sum over the 3 coordinates: each product rounded, summed left to right), then the rebuilt
+# selection_sort_gpu; its first k columns are knn_point's outputs (oracle/gen_golden.py: knn_ref).
 @pytest.mark.parametrize("gen,b,n,m,k", [("U", 4, 4096, 256, 32), ("D", 3, 3000, 200, 32), ("D", 2, 2048, 128, 128), ("S", 2, 1024, 512, 16),
                                          ("U", 2, 40, 10, 40), ("U", 2, 70, 10, 64), ("D", 2, 700, 64, 1), ("U", 1, 8192, 128, 3)])
 def test_knn_point_matches_reference_composite(dev, gen, b, n, m, k):
@@ -126,9 +113,9 @@ def test_knn_point_matches_reference_composite(dev, gen, b, n, m, k):
     x1 = T(xyz, dev)
     x2 = gather_point(x1, farthest_point_sample(m, x1)) if gen != "U" else T(W.cloud_uniform(b, m, 121), dev)
     val, idx = knn_point(k, x1, x2)
-    rval, ridx = _knn_reference_composite(k, x1, x2)
-    assert torch.equal(idx, ridx)
-    assert torch.equal(val, rval)
+    g, case = load_golden("ref_cuda_cases"), f"knn/{gen}_{b}_{n}_{m}_{k}"
+    assert_golden_rows(idx, g, case, "idx")
+    assert_golden_rows(val, g, case, "val")
     with pytest.raises(ValueError):
         knn_point(n + 1, x1, x2)
 
@@ -152,15 +139,13 @@ def test_knn_point_with_nan_and_inf_points_matches_the_selection_sort(dev, k):
     np.testing.assert_array_equal(val.cpu().numpy(), wv)
 
 
-@needs_refcuda
 def test_knn_point_full_size_matches_reference_composite(dev):
-    """(32, 1024, 4096, k = 32) — cfg2's shape, in 4 slices of 8 clouds so that the reference's
-    (b,m,n) matrices stay below 1 GB."""
+    """(32, 1024, 4096, k = 32) — cfg2's shape (the reference composite ran in 4 slices of 8 clouds so
+    that its (b,m,n) matrices stay below 1 GB)."""
     xyz = W.cloud_duplicates(32, 4096, 122)  # ties everywhere
     x1 = T(xyz, dev)
     x2 = gather_point(x1, farthest_point_sample(1024, x1))
     val, idx = knn_point(32, x1, x2)
-    for s in range(0, 32, 8):
-        rval, ridx = _knn_reference_composite(32, x1[s:s + 8].contiguous(), x2[s:s + 8].contiguous())
-        assert torch.equal(idx[s:s + 8], ridx)
-        assert torch.equal(val[s:s + 8], rval)
+    g = load_golden("ref_cuda_cases")
+    assert_golden_rows(idx, g, "knn_full", "idx")
+    assert_golden_rows(val, g, "knn_full", "val")

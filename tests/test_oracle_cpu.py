@@ -1,13 +1,12 @@
 """CPU tests of the oracle itself (no GPU): the C restatement against the reference's own CPU
-functions built from /root/reference (oracle/_ref/libref_cpu.so, when available), the literal FPS
+functions (their outputs on these very inputs, tests/golden/ref_cpu_cases.npz), the literal FPS
 restatement against its closed-form selection order, and the reference's known-answer case."""
 import numpy as np
 import pytest
 
+from conftest import assert_golden_rows, load_golden
 from oracle import oracle as O
 from pointnet2_b200 import workloads as W
-
-needs_refcpu = pytest.mark.skipif(not O.have_refcpu(), reason="oracle/_ref/libref_cpu.so not available")
 
 
 # ---------------------------------------------------------------- FPS restatement
@@ -54,54 +53,49 @@ def test_fps_exhausted_points_emit_index_zero():
 
 
 # ---------------------------------------------------------------- vs the reference's CPU code
-@needs_refcpu
 @pytest.mark.parametrize("r,s", [(0.1, 32), (0.4, 16), (0.05, 8)])
 def test_ball_query_nofma_equals_reference_cpu(r, s):
     xyz = W.cloud_uniform(3, 800, 11)
     new_xyz = O.oracle_gather_point(xyz, O.oracle_fps(100, xyz))
     idx, cnt = O.oracle_query_ball_point(r, s, xyz, new_xyz, use_fma=False)
-    ref = O.refcpu_query_ball_point(r, s, xyz, new_xyz)
-    np.testing.assert_array_equal(idx, ref)
+    assert_golden_rows(idx, load_golden("ref_cpu_cases"), f"bq_nofma/{r}_{s}", "idx")
     assert ((cnt >= 1) & (cnt <= s)).all()  # the centroid itself is always inside its ball
 
 
-@needs_refcpu
 def test_group_point_and_grad_equal_reference_cpu():
+    g = load_golden("ref_cpu_cases")
     xyz = W.cloud_uniform(2, 500, 12)
     feats = W.features(2, 500, 7, 13)
     new_xyz = O.oracle_gather_point(xyz, O.oracle_fps(64, xyz))
     idx, _ = O.oracle_query_ball_point(0.2, 16, xyz, new_xyz)
-    np.testing.assert_array_equal(O.oracle_group_point(feats, idx), O.refcpu_group_point(feats, idx))
+    assert_golden_rows(O.oracle_group_point(feats, idx), g, "group", "out")
     go = W.features(2, 64 * 16, 7, 14).reshape(2, 64, 16, 7)
-    np.testing.assert_array_equal(O.oracle_group_point_grad(feats.shape, idx, go),
-                                  O.refcpu_group_point_grad(feats.shape, idx, go))
+    assert_golden_rows(O.oracle_group_point_grad(feats.shape, idx, go), g, "group_grad", "out")
 
 
-@needs_refcpu
 @pytest.mark.parametrize("n,m,dup", [(600, 150, False), (400, 100, True), (30, 2, False), (10, 1, False)])
 def test_three_nn_equals_reference_cpu(n, m, dup):
+    g = load_golden("ref_cpu_cases")
     xyz1 = W.cloud_duplicates(2, n, 15, drop=False) if dup else W.cloud_uniform(2, n, 15)
     xyz2 = xyz1[:, :m].copy() if dup else W.cloud_uniform(2, m, 16)
     d, i = O.oracle_three_nn(xyz1, xyz2)
-    rd, ri = O.refcpu_three_nn(xyz1, xyz2)
-    np.testing.assert_array_equal(d, rd)
-    np.testing.assert_array_equal(i, ri)
+    assert_golden_rows(d, g, f"three_nn/{n}_{m}_{dup}", "dist")
+    assert_golden_rows(i, g, f"three_nn/{n}_{m}_{dup}", "idx")
     assert (d[:, :, 0] <= d[:, :, 1]).all() and (d[:, :, 1] <= d[:, :, 2]).all()
     if m < 3:
         assert np.isinf(d[:, :, m:]).all() and (i[:, :, m:] == 0).all()
 
 
-@needs_refcpu
 def test_three_interpolate_and_grad_equal_reference_cpu():
+    g = load_golden("ref_cpu_cases")
     xyz1, xyz2 = W.cloud_uniform(2, 300, 17), W.cloud_uniform(2, 60, 18)
     pts = W.features(2, 60, 33, 19)
     d, i = O.oracle_three_nn(xyz1, xyz2)
     dd = np.maximum(d, 1e-10)
     w = ((1.0 / dd) / (1.0 / dd).sum(axis=2, keepdims=True)).astype(np.float32)
-    np.testing.assert_array_equal(O.oracle_three_interpolate(pts, i, w), O.refcpu_three_interpolate(pts, i, w))
+    assert_golden_rows(O.oracle_three_interpolate(pts, i, w), g, "three_interp", "out")
     go = W.features(2, 300, 33, 20)
-    np.testing.assert_array_equal(O.oracle_three_interpolate_grad(pts.shape, i, w, go),
-                                  O.refcpu_three_interpolate_grad(pts.shape, i, w, go))
+    assert_golden_rows(O.oracle_three_interpolate_grad(pts.shape, i, w, go), g, "three_interp_grad", "out")
 
 
 def test_selection_sort_known_answer():

@@ -1,7 +1,8 @@
 """GPU parity tests: the CUDA path (through the ctypes C-ABI) against
   (1) the oracle (CPU restatement) on seeded inputs,
   (2) the committed golden vectors produced by the reference's own kernels (tests/golden/),
-  (3) the reference's own CUDA kernels rebuilt for sm_100a (oracle/_ref/) when they travelled, and
+  (3) the reference's own CUDA kernels rebuilt for sm_100a: their outputs on these tests' inputs
+      (tests/golden/ref_cuda_cases.npz, a seeded sample of rows per case), and
   (4) size-independent properties at BASELINE.json's full sizes.
 Bars: bit-exact for every index tensor and every copied/gathered float; three_interpolate within
 1e-5 abs (it is in fact bit-exact); atomics-based gradients within 1e-4 (the reference's own bar,
@@ -10,7 +11,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import golden_names, load_golden
+from conftest import assert_golden_rows, golden_names, load_golden
 from oracle import oracle as O
 from pointnet2_b200 import _lib, workloads as W
 from pointnet2_b200.tf_grouping import group_point, knn_point, query_ball_point, select_top_k
@@ -105,7 +106,6 @@ def test_fps_cluster_variants_at_full_capacity(dev, cfg, n):
         np.testing.assert_array_equal(N(fx), O.oracle_gather_point(xyz, want))
 
 
-@pytest.mark.skipif(not O.have_refcuda(), reason="oracle/_ref CUDA libraries did not travel")
 @pytest.mark.parametrize("chain", [-1, -2])
 @pytest.mark.parametrize("gen,b,n,m,threads,ppt", [("U", 8, 4096, 1024, 256, 16), ("D", 8, 4096, 1024, 256, 16),
                                                    ("D", 4, 8192, 1024, 256, 32), ("S", 8, 2048, 700, 128, 16),
@@ -114,15 +114,15 @@ def test_fps_both_chains_match_the_reference_kernel(dev, chain, gen, b, n, m, th
     """The plain and the packed chain of the single-CTA kernel against the rebuilt reference kernel at the planner's
     own shapes, every per-thread slot occupied, on clouds with many exact ties (D)."""
     xyz = T(W.DISTRIBUTIONS[gen](b, n, 35), dev)
-    ref = O.refcuda_fps(m, xyz)
+    g, case = load_golden("ref_cuda_cases"), f"fps_chains/{gen}_{b}_{n}_{m}"
     lib = _lib.load()
     lib.pn2_set_fps_config(threads, ppt, chain)
     try:
         fi, fx = farthest_point_sample_and_gather(m, xyz)
     finally:
         lib.pn2_set_fps_config(0, 0, 0)
-    assert torch.equal(fi, ref)
-    assert torch.equal(fx, O.refcuda_gather_point(xyz, ref))
+    assert_golden_rows(fi, g, case, "idx")
+    assert_golden_rows(fx, g, case, "new_xyz")
 
 
 @pytest.mark.parametrize("chain", [-1, -2])
@@ -182,16 +182,16 @@ def test_fps_and_gather_match_reference_golden(dev, name):
     np.testing.assert_array_equal(N(fx), g["new_xyz"])
 
 
-@pytest.mark.skipif(not O.have_refcuda(), reason="oracle/_ref CUDA libraries did not travel")
 @pytest.mark.parametrize("gen,b,n,m", [("U", 8, 4096, 1024), ("D", 4, 8192, 1024), ("S", 32, 1024, 512),
                                        ("U", 2, 16384, 2048), ("D", 1, 65536, 1024)])
 def test_fps_matches_reference_cuda_kernel(dev, gen, b, n, m):
     xyz = T(W.DISTRIBUTIONS[gen](b, n, 33), dev)
-    ref = O.refcuda_fps(m, xyz)
-    assert torch.equal(farthest_point_sample(m, xyz), ref)
+    g, case = load_golden("ref_cuda_cases"), f"fps/{gen}_{b}_{n}_{m}"
+    idx = farthest_point_sample(m, xyz)
+    assert_golden_rows(idx, g, case, "idx")
     fi, fx = farthest_point_sample_and_gather(m, xyz)
-    assert torch.equal(fi, ref)
-    assert torch.equal(fx, O.refcuda_gather_point(xyz, ref))
+    assert torch.equal(fi, idx)
+    assert_golden_rows(fx, g, case, "new_xyz")
 
 
 def test_fps_global_scratch_fallback_matches_oracle(dev):
@@ -379,17 +379,19 @@ def test_ball_query_and_group_match_reference_golden(dev, name):
         np.testing.assert_array_equal(N(group_point(T(g["feats"], dev), idx)), g["grouped_feats"])
 
 
-@pytest.mark.skipif(not O.have_refcuda(), reason="oracle/_ref CUDA libraries did not travel")
 @pytest.mark.parametrize("gen,b,n,m,r,s", [("U", 8, 4096, 1024, 0.1, 32), ("D", 4, 8192, 1024, 0.1, 32),
                                            ("S", 8, 1024, 512, 0.4, 128), ("S", 8, 512, 128, 0.8, 128)])
 def test_ball_query_and_group_match_reference_cuda_kernel(dev, gen, b, n, m, r, s):
     xyz = T(W.DISTRIBUTIONS[gen](b, n, 45), dev)
-    new_xyz = O.refcuda_gather_point(xyz, O.refcuda_fps(m, xyz))
+    g, case = load_golden("ref_cuda_cases"), f"bq/{gen}_{b}_{n}_{m}_{r}_{s}"
+    _, new_xyz = farthest_point_sample_and_gather(m, xyz)  # the reference's centroids (checked below)
+    assert_golden_rows(new_xyz, g, case, "new_xyz")
     idx, cnt = query_ball_point(r, s, xyz, new_xyz)
-    ridx, rcnt = O.refcuda_query_ball_point(r, s, xyz, new_xyz)
-    assert torch.equal(cnt, rcnt)
-    assert torch.equal(idx, ridx)
-    assert torch.equal(group_point(xyz, idx), O.refcuda_group_point(xyz, ridx))
+    assert_golden_rows(cnt, g, case, "cnt")
+    assert_golden_rows(idx, g, case, "idx")
+    grouped = group_point(xyz, idx)
+    assert_golden_rows(grouped, g, case, "grouped")
+    np.testing.assert_array_equal(N(grouped), O.oracle_group_point(N(xyz), N(idx)))
 
 
 def test_ball_query_full_size_properties(dev):
@@ -628,13 +630,14 @@ def test_prob_sample_matches_reference_golden(dev, name):
     np.testing.assert_array_equal(N(temp), g["cumsum"])  # the scratch holds the reference's cumulative sums
 
 
-@pytest.mark.skipif(not O.have_refcuda(), reason="oracle/_ref CUDA libraries did not travel")
 @pytest.mark.parametrize("b,n,m", [(8, 4096, 2048), (2, 100000, 4096), (33, 777, 100)])
 def test_prob_sample_matches_reference_cuda_kernel(dev, b, n, m):
     rng = np.random.RandomState(b + n)
-    p = T(rng.random_sample((b, n)).astype(np.float32), dev)
-    r = T(rng.random_sample((b, m)).astype(np.float32), dev)
-    assert torch.equal(prob_sample(p, r), O.refcuda_prob_sample(p, r))
+    p = rng.random_sample((b, n)).astype(np.float32)
+    r = rng.random_sample((b, m)).astype(np.float32)
+    out = N(prob_sample(T(p, dev), T(r, dev)))
+    assert_golden_rows(out, load_golden("ref_cuda_cases"), f"prob/{b}_{n}_{m}", "out")
+    np.testing.assert_array_equal(out, O.oracle_prob_sample(p, r))
 
 
 def test_prob_sample_rejects_bad_shapes(dev):
