@@ -11,8 +11,10 @@
  *   - plain C, no torch/TF types: sizes are `int`, tensors are raw pointers, `stream` is a
  *     cudaStream_t passed as void* (NULL = legacy default stream, as the reference uses).
  *   - device entry points (pn2_*): every pointer is a DEVICE pointer to a dense row-major
- *     float32 / int32 tensor.  The library allocates nothing, frees nothing and never
- *     synchronises; launches are asynchronous on `stream`.  Stateless and re-entrant.
+ *     float32 / int32 tensor, except the feature pointers of the pn2_*_h entries (`const void*` /
+ *     `void*`), which hold 16-bit features of the type their leading `dtype` names.  The library
+ *     allocates nothing, frees nothing and never synchronises; launches are asynchronous on `stream`.
+ *     Stateless and re-entrant.
  *   - gradients accumulate with float atomics into a buffer the CALLER has zero-filled, exactly
  *     like the reference (tf_sampling.cpp:174, tf_grouping.cpp:204, tf_interpolate.cpp:258).
  *   - return value: 0 on success, otherwise a cudaError_t (argument errors return
@@ -33,6 +35,10 @@ extern "C" {
 #endif
 
 #define PN2_API_VERSION 2
+
+/* feature element types of the pn2_*_h entry points (coordinates and weights are always float32) */
+#define PN2_DTYPE_BF16 1
+#define PN2_DTYPE_F16 2
 
 /* ---- sampling (replaces tf_ops/sampling/tf_sampling_g.cu launchers) ---------------------- */
 
@@ -181,6 +187,37 @@ int pn2_three_nn_interpolate(int b, int n, int m, int c, const float* xyz1, cons
  * points1 (b,n,c1) may be NULL with c1 = 0.  Values equal three_nn -> weights -> three_interpolate -> concat. */
 int pn2_fp_interpolate_concat(int b, int n, int m, int c2, int c1, const float* xyz1, const float* xyz2,
                               const float* points1, const float* points2, float* out, void* stream);
+
+/* ---- 16-bit features: bfloat16 / float16 twins of the feature ops ---------------------------- */
+
+/* Each pn2_*_h entry mirrors the float32 entry named without the suffix, argument for argument, behind a
+ * leading `dtype` (PN2_DTYPE_BF16 or PN2_DTYPE_F16; anything else is cudaErrorInvalidValue).  Feature
+ * tensors (points, points1, points2, out, grad_out) hold that type; xyz, new_xyz, xyz1, xyz2, weight,
+ * dist and grouped_xyz stay float32.  Values: every output equals the float32 op applied to the features
+ * widened exactly to float32, rounded once to nearest-even into `dtype` (gathers and concats copy bits).
+ * Gradients read a 16-bit grad_out and write FLOAT32 grad_points: the atomic entries accumulate into a
+ * buffer the caller has zero-filled, the _det entry overwrites (same workspace size as its float32 twin,
+ * and bit-identical to it applied to grad_out widened to float32). */
+int pn2_group_point_h(int dtype, int b, int n, int c, int m, int nsample, const void* points, const int* idx,
+                      void* out, void* stream);
+int pn2_group_point_grad_h(int dtype, int b, int n, int c, int m, int nsample, const void* grad_out,
+                           const int* idx, float* grad_points, void* stream);
+int pn2_group_concat_h(int dtype, int b, int n, int c, int m, int nsample, const float* xyz, const float* new_xyz,
+                       const void* points, const int* idx, int xyz_first, void* out, float* grouped_xyz,
+                       void* stream);
+int pn2_three_interpolate_h(int dtype, int b, int m, int c, int n, const void* points, const int* idx,
+                            const float* weight, void* out, void* stream);
+int pn2_three_interpolate_grad_h(int dtype, int b, int n, int c, int m, const void* grad_out, const int* idx,
+                                 const float* weight, float* grad_points, void* stream);
+int pn2_three_interpolate_grad_det_h(int dtype, int b, int n, int c, int m, const void* grad_out, const int* idx,
+                                     const float* weight, float* grad_points, void* workspace,
+                                     size_t workspace_bytes, void* stream);
+int pn2_three_nn_interpolate_h(int dtype, int b, int n, int m, int c, const float* xyz1, const float* xyz2,
+                               const void* points2, void* out, float* dist, int* idx, float* weight,
+                               void* stream);
+int pn2_fp_interpolate_concat_h(int dtype, int b, int n, int m, int c2, int c1, const float* xyz1,
+                                const float* xyz2, const void* points1, const void* points2, void* out,
+                                void* stream);
 
 /* ---- the sampling+grouping half of a set-abstraction layer, device-resident ------------------ */
 

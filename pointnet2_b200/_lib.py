@@ -38,6 +38,15 @@ _SIGNATURES = {
     "pn2_fp_interpolate_concat": (c_int, [c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     "pn2_group_concat": (c_int, [c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, c_int, _P, _P, _P]),
     "pn2_three_nn_interpolate": (c_int, [c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, _P]),
+    # 16-bit features: leading dtype code (PN2_DTYPE_BF16 / PN2_DTYPE_F16), then the float32 twin's arguments
+    "pn2_group_point_h": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P]),
+    "pn2_group_point_grad_h": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P]),
+    "pn2_group_concat_h": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, c_int, _P, _P, _P]),
+    "pn2_three_interpolate_h": (c_int, [c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P]),
+    "pn2_three_interpolate_grad_h": (c_int, [c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P]),
+    "pn2_three_interpolate_grad_det_h": (c_int, [c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, c_size_t, _P]),
+    "pn2_three_nn_interpolate_h": (c_int, [c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "pn2_fp_interpolate_concat_h": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     "pn2_ball_group_fits": (c_int, [c_int]),
     "pn2_ball_group": (c_int, [c_int, c_int, c_int, c_float, c_int, _P, _P, _P, _P, _P, c_int, _P]),
     "pn2_sa_layer_device_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),

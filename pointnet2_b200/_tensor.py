@@ -24,6 +24,22 @@ def require_cuda(t: torch.Tensor, name: str, dtype: torch.dtype) -> torch.Tensor
     return t if t.is_contiguous() else t.contiguous()
 
 
+# feature dtypes and their codes in the C ABI (include/pn2_api.h: PN2_DTYPE_BF16, PN2_DTYPE_F16; 0 = float32, which
+# calls the float32 entry points)
+FEATURE_DTYPES = {torch.float32: 0, torch.bfloat16: 1, torch.float16: 2}
+
+
+def feature_dtype_code(t, name: str) -> int:
+    """Features may be float32, bfloat16 or float16 (coordinates and weights stay float32): the ABI dtype code of
+    ``t``, TypeError for anything else."""
+    if not isinstance(t, torch.Tensor):
+        raise TypeError(f"{name} must be a torch.Tensor, got {type(t).__name__}")
+    code = FEATURE_DTYPES.get(t.dtype)
+    if code is None:
+        raise TypeError(f"{name} must be torch.float32, torch.bfloat16 or torch.float16, got {t.dtype}")
+    return code
+
+
 def same_device(*ts: torch.Tensor) -> None:
     dev = ts[0].device
     for t in ts[1:]:

@@ -464,6 +464,254 @@ static unsigned grid_for(unsigned long long work_items, unsigned per_block) {
 }
 
 
+// ---- 16-bit features (pn2_*_h) -------------------------------------------------------------------
+// A gather copies bits, so pn2_group_point_h hands every layout the float32 kernels already move — c even with
+// 4-byte aligned bases: rows of c/2 words, float4 rows when c % 8 == 0 — to pn2_group_point.  What is left here:
+// odd c / 2-byte aligned rows, and the concat tail, whose centred xyz is computed in float32 and rounded once.
+// group_rows_h_kernel is group_rows_kernel with 2-byte elements (U = 8: the same bytes in flight per lane).
+template <int LPR, bool HAS_XYZ, int DT>
+__global__ void __launch_bounds__(kCopyThreads)
+group_rows_h_kernel(int n, int c, int nsample, unsigned rows_per_cloud, const float* __restrict__ xyz,
+                    const float* __restrict__ new_xyz, const unsigned short* __restrict__ points,
+                    const int* __restrict__ idx, int xyz_lo, int feat_lo, unsigned short* __restrict__ out,
+                    float* __restrict__ grouped_xyz) {
+    constexpr int RPW = 32 / LPR;
+    const int lane = threadIdx.x & 31, g = lane % LPR, sub = lane / LPR;
+    const unsigned cloud = blockIdx.y;
+    const int w = c + (HAS_XYZ ? 3 : 0);
+    const unsigned warps = (gridDim.x * kCopyThreads) >> 5;
+    const unsigned warp = (blockIdx.x * kCopyThreads + threadIdx.x) >> 5;
+    const size_t cloud_row0 = (size_t)cloud * rows_per_cloud;
+    const int* __restrict__ cidx = idx + cloud_row0;
+    const unsigned short* __restrict__ cpts = points ? points + (size_t)cloud * n * c : nullptr;
+    const float* __restrict__ cxyz = HAS_XYZ ? xyz + (size_t)cloud * n * 3 : nullptr;
+    constexpr int R = 2, U = 8;
+    for (unsigned r0 = (warp * RPW + sub) * R; r0 < rows_per_cloud; r0 += warps * RPW * R) {
+        const unsigned short* __restrict__ src[R];
+        unsigned short* __restrict__ d[R];
+        bool ok[R];
+#pragma unroll
+        for (int rr = 0; rr < R; ++rr) {
+            const unsigned r = r0 + rr;
+            ok[rr] = r < rows_per_cloud;
+            const int a = ok[rr] ? __ldg(cidx + r) : 0;
+            unsigned short* __restrict__ dst = out + (cloud_row0 + r) * w;
+            src[rr] = cpts ? cpts + (size_t)a * c : nullptr;
+            d[rr] = dst + feat_lo;
+            if (HAS_XYZ && ok[rr] && g < 3) {
+                const size_t ctr = (size_t)cloud * (rows_per_cloud / (unsigned)nsample) + r / (unsigned)nsample;
+                const float v = __fsub_rn(__ldg(cxyz + (size_t)a * 3 + g), __ldg(new_xyz + ctr * 3 + g));
+                __stcs(dst + xyz_lo + g, f_to_h<DT>(v));
+                if (grouped_xyz) __stcs(grouped_xyz + (cloud_row0 + r) * 3 + g, v);
+            }
+        }
+        for (int l0 = g; l0 < c; l0 += LPR * U) {
+            unsigned short v[R][U];
+#pragma unroll
+            for (int rr = 0; rr < R; ++rr)
+#pragma unroll
+                for (int u = 0; u < U; ++u)
+                    if (ok[rr] && l0 + u * LPR < c) v[rr][u] = __ldg(src[rr] + l0 + u * LPR);
+#pragma unroll
+            for (int rr = 0; rr < R; ++rr)
+#pragma unroll
+                for (int u = 0; u < U; ++u)
+                    if (ok[rr] && l0 + u * LPR < c) __stcs(d[rr] + l0 + u * LPR, v[rr][u]);
+        }
+    }
+}
+
+// The concat tail with 16-bit features, c % 8 == 0: 16-byte gathers of 8 values AND 16-byte stores.  Output rows are
+// 3 + c values wide, so a row's feature segment starts `head` = 0..7 values before a 16-byte boundary, differently
+// for every row.  As in group_concat_vec_kernel, lane k loads source vector k, gets vector k+1 from its neighbour
+// (the last lane of a pass loads it), and stores the aligned output vector that starts `head` values into the
+// segment: words q = head/2 .. q+4 of the pair, funnel-shifted by 16 bits when head is odd.  The head values, the
+// 8 - head tail values and the 3 centred xyz of a row are scalar stores.  R rows' gathers are in flight before the
+// first store.
+template <int LPR, int R, int DT>
+__global__ void __launch_bounds__(kCopyThreads, 4)
+group_concat_h_vec_kernel(int n, int c8, int nsample, unsigned rows_per_cloud, const float* __restrict__ xyz,
+                          const float* __restrict__ new_xyz, const uint4* __restrict__ points, const int* __restrict__ idx,
+                          int xyz_lo, int feat_lo, unsigned short* __restrict__ out, float* __restrict__ grouped_xyz) {
+    constexpr int RPW = 32 / LPR;
+    const int lane = threadIdx.x & 31, g = lane % LPR, sub = lane / LPR;
+    const unsigned cloud = blockIdx.y;
+    const unsigned warps = (gridDim.x * kCopyThreads) >> 5;
+    const unsigned warp = (blockIdx.x * kCopyThreads + threadIdx.x) >> 5;
+    const size_t cloud_row0 = (size_t)cloud * rows_per_cloud;
+    const unsigned m = rows_per_cloud / (unsigned)nsample;
+    const int c = 8 * c8;
+    const size_t w = (size_t)c + 3;
+    const int* __restrict__ cidx = idx + cloud_row0;
+    const uint4* __restrict__ cpts = points + (size_t)cloud * n * c8;
+    const float* __restrict__ cxyz = xyz + (size_t)cloud * n * 3;
+    const float* __restrict__ cctr = new_xyz + (size_t)cloud * m * 3;
+    for (unsigned r0 = (warp * RPW + sub) * R; r0 < rows_per_cloud; r0 += warps * RPW * R) {
+        const uint4* __restrict__ src[R];
+        unsigned short* __restrict__ fdst[R];
+        int head[R];
+        bool ok[R];
+#pragma unroll
+        for (int rr = 0; rr < R; ++rr) {
+            const unsigned r = r0 + rr;
+            ok[rr] = r < rows_per_cloud;
+            const int a = ok[rr] ? __ldg(cidx + r) : 0;
+            src[rr] = cpts + (size_t)a * c8;
+            const size_t obase = (cloud_row0 + r) * w;
+            fdst[rr] = out + obase + feat_lo;
+            head[rr] = (int)((8u - (unsigned)((obase + (size_t)feat_lo) & 7u)) & 7u);
+            // scalar slots: t < 3 the centred xyz, then head value t-3 or tail value c-8+(t-3) (11 slots)
+            if (ok[rr]) {
+                for (int t = g; t < 11; t += LPR) {
+                    const int h = head[rr];
+                    if (t < 3) {
+                        const float val =
+                            __fsub_rn(__ldg(cxyz + (size_t)a * 3 + t), __ldg(cctr + (size_t)(r / (unsigned)nsample) * 3 + t));
+                        __stcs(out + obase + xyz_lo + t, f_to_h<DT>(val));
+                        if (grouped_xyz) __stcs(grouped_xyz + (cloud_row0 + r) * 3 + t, val);
+                    } else if (h != 0) {
+                        const int e = t - 3 < h ? t - 3 : c - 8 + (t - 3);
+                        __stcs(fdst[rr] + e, __ldg(reinterpret_cast<const unsigned short*>(src[rr]) + e));
+                    }
+                }
+            }
+        }
+        for (int k0 = 0; k0 < c8; k0 += LPR) {
+            const int k = k0 + g;
+            uint4 v[R], nx[R];
+#pragma unroll
+            for (int rr = 0; rr < R; ++rr) {
+                v[rr] = make_uint4(0u, 0u, 0u, 0u);
+                if (ok[rr] && k < c8) v[rr] = __ldg(src[rr] + k);
+            }
+#pragma unroll
+            for (int rr = 0; rr < R; ++rr) {
+                nx[rr].x = __shfl_down_sync(kFullMask, v[rr].x, 1, LPR);
+                nx[rr].y = __shfl_down_sync(kFullMask, v[rr].y, 1, LPR);
+                nx[rr].z = __shfl_down_sync(kFullMask, v[rr].z, 1, LPR);
+                nx[rr].w = __shfl_down_sync(kFullMask, v[rr].w, 1, LPR);
+                if (g == LPR - 1 && ok[rr] && k + 1 < c8 && head[rr] != 0) nx[rr] = __ldg(src[rr] + k + 1);
+            }
+#pragma unroll
+            for (int rr = 0; rr < R; ++rr) {
+                if (!ok[rr] || k >= c8) continue;
+                const int h = head[rr];
+                unsigned short* __restrict__ d = fdst[rr];
+                if (h == 0) {
+                    __stcs(reinterpret_cast<uint4*>(d) + k, v[rr]);
+                    continue;
+                }
+                if (k + 1 < c8) {  // values [h + 8k, h + 8k + 8) of the segment
+                    const unsigned W[8] = {v[rr].x, v[rr].y, v[rr].z, v[rr].w, nx[rr].x, nx[rr].y, nx[rr].z, nx[rr].w};
+                    const int q = h >> 1;
+                    const unsigned sh = (unsigned)(h & 1) * 16u;
+                    unsigned s5[5];
+#pragma unroll
+                    for (int i = 0; i < 5; ++i) s5[i] = q == 0 ? W[i] : (q == 1 ? W[i + 1] : (q == 2 ? W[i + 2] : W[i + 3]));
+                    uint4 o;
+                    o.x = __funnelshift_r(s5[0], s5[1], sh);
+                    o.y = __funnelshift_r(s5[1], s5[2], sh);
+                    o.z = __funnelshift_r(s5[2], s5[3], sh);
+                    o.w = __funnelshift_r(s5[3], s5[4], sh);
+                    __stcs(reinterpret_cast<uint4*>(d + h + 8 * k), o);
+                }
+            }
+        }
+    }
+}
+
+template <bool HAS_XYZ, int DT>
+static int launch_group_rows_h(int b, int n, int c, int m, int nsample, const float* xyz, const float* new_xyz,
+                               const unsigned short* points, const int* idx, int xyz_lo, int feat_lo, unsigned short* out,
+                               float* grouped_xyz, cudaStream_t st) {
+    const unsigned rpc = (unsigned)m * (unsigned)nsample;
+    const unsigned cap = (148u * 32u + b - 1) / b;  // enough CTAs to fill the machine, then grid-stride
+    if (HAS_XYZ && c > 0 && c % 8 == 0 && aligned16(points) && aligned16(out)) {
+        const int c8 = c / 8;
+        // lanes per row: the widest that leaves the fewest lanes idle in the row's last pass (C = 320: 40 vectors
+        // are 5 full passes of 8 lanes, not 32 + 8 of 32 lanes)
+        int lpr = 8;
+        for (int l = 16; l <= 32; l *= 2)
+            if ((c8 + l - 1) / l * l <= (c8 + lpr - 1) / lpr * lpr) lpr = l;
+        constexpr int R = 2;
+        const unsigned rows_per_block = (kCopyThreads / 32) * (32 / lpr) * R;
+        unsigned gx = (rpc + rows_per_block - 1) / rows_per_block;
+        if (gx > cap) gx = cap;
+        if (gx < 1) gx = 1;
+        dim3 grid(gx, b, 1);
+        const uint4* p8 = reinterpret_cast<const uint4*>(points);
+        if (lpr == 8) group_concat_h_vec_kernel<8, R, DT><<<grid, kCopyThreads, 0, st>>>(n, c8, nsample, rpc, xyz, new_xyz, p8, idx, xyz_lo, feat_lo, out, grouped_xyz);
+        else if (lpr == 16) group_concat_h_vec_kernel<16, R, DT><<<grid, kCopyThreads, 0, st>>>(n, c8, nsample, rpc, xyz, new_xyz, p8, idx, xyz_lo, feat_lo, out, grouped_xyz);
+        else group_concat_h_vec_kernel<32, R, DT><<<grid, kCopyThreads, 0, st>>>(n, c8, nsample, rpc, xyz, new_xyz, p8, idx, xyz_lo, feat_lo, out, grouped_xyz);
+        return finish_launch();
+    }
+    const int w = c + (HAS_XYZ ? 3 : 0);
+    const int lpr = w <= 4 ? 4 : (w <= 8 ? 8 : (w <= 16 ? 16 : 32));
+    const unsigned rows_per_block = (kCopyThreads / 32) * (32 / lpr) * 2;
+    unsigned gx = (rpc + rows_per_block - 1) / rows_per_block;
+    if (gx > cap) gx = cap;
+    if (gx < 1) gx = 1;
+    dim3 grid(gx, b, 1);
+#define PN2_GROUP_ROWS_H(L) \
+    group_rows_h_kernel<L, HAS_XYZ, DT><<<grid, kCopyThreads, 0, st>>>(n, c, nsample, rpc, xyz, new_xyz, points, idx, xyz_lo, feat_lo, out, grouped_xyz)
+    if (lpr == 4) PN2_GROUP_ROWS_H(4);
+    else if (lpr == 8) PN2_GROUP_ROWS_H(8);
+    else if (lpr == 16) PN2_GROUP_ROWS_H(16);
+    else PN2_GROUP_ROWS_H(32);
+#undef PN2_GROUP_ROWS_H
+    return finish_launch();
+}
+
+// group_point_grad with a 16-bit grad_out: widened exactly, float atomics into float32 grad_points.  VEC: 4 channels
+// per thread (8-byte loads, red.global.add.v4.f32), c % 4 == 0.
+template <typename IndexT, int DT, bool VEC>
+__global__ void __launch_bounds__(kCopyThreads)
+group_point_grad_h_kernel(int n, int c, IndexT rows_per_cloud, IndexT total, const unsigned short* __restrict__ grad_out,
+                          const int* __restrict__ idx, float* __restrict__ grad_points) {
+    constexpr int W = VEC ? 4 : 1;
+    const int cw = c / W;
+    const IndexT stride = (IndexT)gridDim.x * kCopyThreads;
+    for (IndexT e = (IndexT)blockIdx.x * kCopyThreads + threadIdx.x; e < total; e += stride) {
+        const IndexT row = e / (IndexT)cw;
+        const int l = (int)(e - row * (IndexT)cw) * W;
+        const IndexT cloud = row / rows_per_cloud;
+        const int a = __ldg(idx + row);
+        float* gp = grad_points + ((size_t)cloud * n + a) * c + l;
+        if (VEC) {
+            const uint2 u = __ldcs(reinterpret_cast<const uint2*>(grad_out) + e);
+            const float2 lo = h2_to_f2<DT>(u.x), hi = h2_to_f2<DT>(u.y);
+            atomicAdd(reinterpret_cast<float4*>(gp), make_float4(lo.x, lo.y, hi.x, hi.y));
+        } else {
+            atomicAdd(gp, h_to_f<DT>(__ldcs(grad_out + e)));
+        }
+    }
+}
+
+template <int DT>
+static int group_point_grad_h(int b, int n, int c, int m, int nsample, const unsigned short* grad_out, const int* idx,
+                              float* grad_points, cudaStream_t st) {
+    const unsigned long long rpc = (unsigned long long)m * nsample;
+    const unsigned long long total = (unsigned long long)b * rpc * c;
+    if (c % 4 == 0 && (reinterpret_cast<uintptr_t>(grad_out) & 7u) == 0 && aligned16(grad_points)) {
+        const unsigned long long tv = total / 4;
+        const unsigned grid = grid_for(tv, kCopyThreads);
+        if (tv < (1ull << 31))
+            group_point_grad_h_kernel<unsigned, DT, true><<<grid, kCopyThreads, 0, st>>>(n, c, (unsigned)rpc, (unsigned)tv, grad_out, idx, grad_points);
+        else
+            group_point_grad_h_kernel<unsigned long long, DT, true><<<grid, kCopyThreads, 0, st>>>(n, c, rpc, tv, grad_out, idx, grad_points);
+    } else {
+        const unsigned grid = grid_for(total, kCopyThreads);
+        if (total < (1ull << 31))
+            group_point_grad_h_kernel<unsigned, DT, false><<<grid, kCopyThreads, 0, st>>>(n, c, (unsigned)rpc, (unsigned)total, grad_out, idx, grad_points);
+        else
+            group_point_grad_h_kernel<unsigned long long, DT, false><<<grid, kCopyThreads, 0, st>>>(n, c, rpc, total, grad_out, idx, grad_points);
+    }
+    return finish_launch();
+}
+
+static bool aligned4(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 3u) == 0; }
+
+
 }  // namespace pn2
 
 extern "C" {
@@ -590,6 +838,51 @@ int pn2_selection_sort(int b, int n, int m, int k, const float* dist, int* outi,
     if (blocks > 0x7fffffffull) return (int)cudaErrorInvalidValue;
     selection_sort_kernel<<<(unsigned)blocks, kCopyThreads, 0, as_stream(stream)>>>(n, k, rows, dist, outi, out);
     return finish_launch();
+}
+
+int pn2_group_point_h(int dtype, int b, int n, int c, int m, int nsample, const void* points, const int* idx, void* out,
+                      void* stream) {
+    using namespace pn2;
+    if (!valid_half_dtype(dtype)) return (int)cudaErrorInvalidValue;
+    if (b < 0 || n <= 0 || c < 0 || m < 0 || nsample < 0) return (int)cudaErrorInvalidValue;
+    const unsigned long long rpc = (unsigned long long)m * nsample;
+    if ((unsigned long long)b * rpc * c == 0) return 0;
+    if (!points || !idx || !out) return (int)cudaErrorInvalidValue;
+    // the bytes do not depend on the element type: even rows on 4-byte aligned bases are rows of c/2 float32 words
+    if (c % 2 == 0 && aligned4(points) && aligned4(out))
+        return pn2_group_point(b, n, c / 2, m, nsample, static_cast<const float*>(points), idx, static_cast<float*>(out), stream);
+    if (rpc >= (1ull << 32) || b > 65535) return (int)cudaErrorInvalidValue;
+    return launch_group_rows_h<false, PN2_DTYPE_BF16>(b, n, c, m, nsample, nullptr, nullptr, static_cast<const unsigned short*>(points),
+                                                      idx, 0, 0, static_cast<unsigned short*>(out), nullptr, as_stream(stream));
+}
+
+int pn2_group_point_grad_h(int dtype, int b, int n, int c, int m, int nsample, const void* grad_out, const int* idx,
+                           float* grad_points, void* stream) {
+    using namespace pn2;
+    if (!valid_half_dtype(dtype)) return (int)cudaErrorInvalidValue;
+    if (b < 0 || n <= 0 || c < 0 || m < 0 || nsample < 0) return (int)cudaErrorInvalidValue;
+    if ((unsigned long long)b * m * nsample * c == 0) return 0;
+    if (!grad_out || !idx || !grad_points) return (int)cudaErrorInvalidValue;
+    const unsigned short* g = static_cast<const unsigned short*>(grad_out);
+    if (dtype == PN2_DTYPE_BF16) return group_point_grad_h<PN2_DTYPE_BF16>(b, n, c, m, nsample, g, idx, grad_points, as_stream(stream));
+    return group_point_grad_h<PN2_DTYPE_F16>(b, n, c, m, nsample, g, idx, grad_points, as_stream(stream));
+}
+
+int pn2_group_concat_h(int dtype, int b, int n, int c, int m, int nsample, const float* xyz, const float* new_xyz,
+                       const void* points, const int* idx, int xyz_first, void* out, float* grouped_xyz, void* stream) {
+    using namespace pn2;
+    if (!valid_half_dtype(dtype)) return (int)cudaErrorInvalidValue;
+    if (b < 0 || n <= 0 || c < 0 || m < 0 || nsample < 0) return (int)cudaErrorInvalidValue;
+    const unsigned long long rpc = (unsigned long long)m * nsample;
+    if (b == 0 || rpc == 0) return 0;
+    if (!xyz || !new_xyz || !idx || !out || (c > 0 && !points)) return (int)cudaErrorInvalidValue;
+    if (rpc >= (1ull << 32) || b > 65535) return (int)cudaErrorInvalidValue;
+    const int xyz_lo = xyz_first ? 0 : c, feat_lo = xyz_first ? 3 : 0;
+    const unsigned short* p = static_cast<const unsigned short*>(points);
+    unsigned short* o = static_cast<unsigned short*>(out);
+    if (dtype == PN2_DTYPE_BF16)
+        return launch_group_rows_h<true, PN2_DTYPE_BF16>(b, n, c, m, nsample, xyz, new_xyz, p, idx, xyz_lo, feat_lo, o, grouped_xyz, as_stream(stream));
+    return launch_group_rows_h<true, PN2_DTYPE_F16>(b, n, c, m, nsample, xyz, new_xyz, p, idx, xyz_lo, feat_lo, o, grouped_xyz, as_stream(stream));
 }
 
 }  // extern "C"

@@ -166,6 +166,18 @@ __device__ __forceinline__ float interp3(float p1, float p2, float p3, float w1,
     return __fadd_rn(__fadd_rn(__fmul_rn(p1, w1), __fmul_rn(p2, w2)), __fmul_rn(p3, w3));
 }
 
+// 8 16-bit values of each of three rows (16-byte vectors): widened exactly, interp3, one rounding each
+template <int DT>
+__device__ __forceinline__ unsigned interp3_h2(unsigned a, unsigned b, unsigned c, float w1, float w2, float w3) {
+    const float2 x = h2_to_f2<DT>(a), y = h2_to_f2<DT>(b), z = h2_to_f2<DT>(c);
+    return f2_to_h2<DT>(interp3(x.x, y.x, z.x, w1, w2, w3), interp3(x.y, y.y, z.y, w1, w2, w3));
+}
+template <int DT>
+__device__ __forceinline__ uint4 interp3_h8(uint4 a, uint4 b, uint4 c, float w1, float w2, float w3) {
+    return make_uint4(interp3_h2<DT>(a.x, b.x, c.x, w1, w2, w3), interp3_h2<DT>(a.y, b.y, c.y, w1, w2, w3),
+                      interp3_h2<DT>(a.z, b.z, c.z, w1, w2, w3), interp3_h2<DT>(a.w, b.w, c.w, w1, w2, w3));
+}
+
 constexpr int kItThreads = 256;
 
 // One thread per output float4 (U = 1).  Measured in round 2 (profiles/r2_interp_experiments.txt): U = 4 outputs in
@@ -303,6 +315,46 @@ __device__ __forceinline__ void top3_insert_lex(Top3& t, float d, int k) {
     t.i1 = c1 ? k : t.i1;
 }
 
+// Phase 2 of fp_front_kernel for 16-bit features: 16-byte loads of 8 values when c2 and c1 are multiples of 8 and the
+// rows are 16-byte aligned, else one value per lane.
+template <int DT, int PPB>
+__device__ __forceinline__ void fp_front_phase2_h(int rows, int c2, int c1, const unsigned short* __restrict__ pb,
+                                                  const unsigned short* __restrict__ p1, unsigned short* __restrict__ ob,
+                                                  const int (&s_i)[PPB][3], const float (&s_w)[PPB][3], int tid) {
+    const int cw = c2 + c1;
+    const bool vec = ((c2 | c1) & 7) == 0 &&
+                     ((reinterpret_cast<uintptr_t>(pb) | reinterpret_cast<uintptr_t>(ob) | reinterpret_cast<uintptr_t>(p1)) & 15u) == 0;
+    if (vec) {
+        const int c28 = c2 >> 3, cw8 = cw >> 3, c18 = c1 >> 3;
+        const uint4* pb8 = reinterpret_cast<const uint4*>(pb);
+        const uint4* p18 = reinterpret_cast<const uint4*>(p1);
+        uint4* ob8 = reinterpret_cast<uint4*>(ob);
+        for (int e = tid; e < rows * cw8; e += kNnThreads) {
+            const int r = e / cw8, l = e - r * cw8;
+            uint4 o;
+            if (l < c28) {
+                const uint4 a = __ldg(pb8 + (size_t)s_i[r][0] * c28 + l), b = __ldg(pb8 + (size_t)s_i[r][1] * c28 + l),
+                            cc = __ldg(pb8 + (size_t)s_i[r][2] * c28 + l);
+                o = interp3_h8<DT>(a, b, cc, s_w[r][0], s_w[r][1], s_w[r][2]);
+            } else {
+                o = __ldcs(p18 + (size_t)r * c18 + (l - c28));
+            }
+            __stcs(ob8 + e, o);
+        }
+    } else {
+        for (int e = tid; e < rows * cw; e += kNnThreads) {
+            const int r = e / cw, l = e - r * cw;
+            unsigned short o;
+            if (l < c2)
+                o = f_to_h<DT>(interp3(h_to_f<DT>(__ldg(pb + (size_t)s_i[r][0] * c2 + l)), h_to_f<DT>(__ldg(pb + (size_t)s_i[r][1] * c2 + l)),
+                                       h_to_f<DT>(__ldg(pb + (size_t)s_i[r][2] * c2 + l)), s_w[r][0], s_w[r][1], s_w[r][2]));
+            else
+                o = __ldcs(p1 + (size_t)r * c1 + (l - c2));
+            ob[e] = o;
+        }
+    }
+}
+
 // lane g of G scans pairs g, g+G, ... of the tile (2 points per pair)
 template <int G>
 __device__ __forceinline__ void scan_tile_strided(Top3& t, const KnownTile& tile, int tp_pad, int base, int g, float ux, float uy,
@@ -322,10 +374,12 @@ __device__ __forceinline__ void scan_tile_strided(Top3& t, const KnownTile& tile
     }
 }
 
-template <int G>
+// DT: feature type of points1 / points2 / out (0 = float32, or PN2_DTYPE_BF16 / PN2_DTYPE_F16: values widened exactly,
+// interp3 in float32, one rounding); phase 1 does not depend on it.
+template <int G, int DT>
 __global__ void __launch_bounds__(kNnThreads)
 fp_front_kernel(int n, int m, int c2, int c1, const float* __restrict__ xyz1, const float* __restrict__ xyz2,
-                const float* __restrict__ points1, const float* __restrict__ points2, float* __restrict__ out,
+                const feat_t<DT>* __restrict__ points1, const feat_t<DT>* __restrict__ points2, feat_t<DT>* __restrict__ out,
                 float* __restrict__ dist_o, int* __restrict__ idx_o, float* __restrict__ weight_o) {
     constexpr int PPB = kNnThreads / G;  // unknown points per CTA
     __shared__ KnownTile s_tile;
@@ -387,9 +441,13 @@ fp_front_kernel(int n, int m, int c2, int c1, const float* __restrict__ xyz1, co
     if (!out) return;
     const int rows = min(PPB, n - j0);
     const int cw = c2 + c1;  // output row width
-    const float* __restrict__ pb = points2 + (size_t)cloud * m * c2;
-    const float* __restrict__ p1 = points1 ? points1 + ((size_t)cloud * n + j0) * c1 : nullptr;
-    float* __restrict__ ob = out + ((size_t)cloud * n + j0) * cw;
+    const feat_t<DT>* __restrict__ pb = points2 + (size_t)cloud * m * c2;
+    const feat_t<DT>* __restrict__ p1 = points1 ? points1 + ((size_t)cloud * n + j0) * c1 : nullptr;
+    feat_t<DT>* __restrict__ ob = out + ((size_t)cloud * n + j0) * cw;
+    if constexpr (DT != 0) {
+        fp_front_phase2_h<DT>(rows, c2, c1, pb, p1, ob, s_i, s_w, tid);
+        return;
+    } else {
     const bool vec = ((c2 | c1) & 3) == 0 &&
                      ((reinterpret_cast<uintptr_t>(pb) | reinterpret_cast<uintptr_t>(ob) | reinterpret_cast<uintptr_t>(p1)) & 15u) == 0;
     if (vec) {
@@ -425,31 +483,33 @@ fp_front_kernel(int n, int m, int c2, int c1, const float* __restrict__ xyz1, co
             ob[e] = o;
         }
     }
+    }
 }
 
-template <int G>
-static int launch_fp_front(int b, int n, int m, int c2, int c1, const float* xyz1, const float* xyz2, const float* points1,
-                           const float* points2, float* out, float* dist, int* idx, float* weight, cudaStream_t st) {
+template <int G, int DT>
+static int launch_fp_front(int b, int n, int m, int c2, int c1, const float* xyz1, const float* xyz2, const feat_t<DT>* points1,
+                           const feat_t<DT>* points2, feat_t<DT>* out, float* dist, int* idx, float* weight, cudaStream_t st) {
     constexpr int PPB = kNnThreads / G;
     dim3 grid((n + PPB - 1) / PPB, b, 1);
-    fp_front_kernel<G><<<grid, kNnThreads, 0, st>>>(n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight);
+    fp_front_kernel<G, DT><<<grid, kNnThreads, 0, st>>>(n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight);
     return finish_launch();
 }
 
-static int fp_front_dispatch(int b, int n, int m, int c2, int c1, const float* xyz1, const float* xyz2, const float* points1,
-                             const float* points2, float* out, float* dist, int* idx, float* weight, cudaStream_t st) {
+template <int DT>
+static int fp_front_dispatch(int b, int n, int m, int c2, int c1, const float* xyz1, const float* xyz2, const feat_t<DT>* points1,
+                             const feat_t<DT>* points2, feat_t<DT>* out, float* dist, int* idx, float* weight, cudaStream_t st) {
     // lanes per unknown point: as many as it takes to put ~2 CTAs on every SM (a CTA covers 128/G points),
     // but never more lanes than there are pairs of known points to share
     const long long pts = (long long)b * n;
     int G = 1;
     while (G < 32 && pts * G < 2LL * 148 * kNnThreads && 2 * G <= (m + 1) / 2) G *= 2;
     switch (G) {
-        case 1: return launch_fp_front<1>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
-        case 2: return launch_fp_front<2>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
-        case 4: return launch_fp_front<4>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
-        case 8: return launch_fp_front<8>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
-        case 16: return launch_fp_front<16>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
-        default: return launch_fp_front<32>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
+        case 1: return launch_fp_front<1, DT>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
+        case 2: return launch_fp_front<2, DT>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
+        case 4: return launch_fp_front<4, DT>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
+        case 8: return launch_fp_front<8, DT>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
+        case 16: return launch_fp_front<16, DT>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
+        default: return launch_fp_front<32, DT>(b, n, m, c2, c1, xyz1, xyz2, points1, points2, out, dist, idx, weight, st);
     }
 }
 
@@ -570,11 +630,28 @@ inv_build_kernel(int n3, int m, const int* __restrict__ idx, int* __restrict__ o
     for (int e = tid; e < n3; e += 1024) ent[atomicAdd(&s_c[__ldg(cidx + e)], 1)] = e;
 }
 
-// one warp per known point (b, i); lanes over channels (float4 when VEC).  Lists longer than kInvSortCap are
-// queued for inv_long_kernel.
-template <bool VEC>
+// 4 consecutive entries / one entry of grad_out, widened exactly to float32 (DT = 0: float32 grad_out)
+template <int DT>
+__device__ __forceinline__ float4 ld_grad4(const feat_t<DT>* __restrict__ p) {
+    if constexpr (DT == 0) {
+        return __ldg(reinterpret_cast<const float4*>(p));
+    } else {
+        const uint2 u = __ldg(reinterpret_cast<const uint2*>(p));
+        const float2 lo = h2_to_f2<DT>(u.x), hi = h2_to_f2<DT>(u.y);
+        return make_float4(lo.x, lo.y, hi.x, hi.y);
+    }
+}
+template <int DT>
+__device__ __forceinline__ float ld_grad1(const feat_t<DT>* __restrict__ p) {
+    if constexpr (DT == 0) return __ldg(p);
+    else return h_to_f<DT>(__ldg(p));
+}
+
+// one warp per known point (b, i); lanes over channels (4 channels per lane when VEC).  Lists longer than kInvSortCap
+// are queued for inv_long_kernel.  DT: grad_out's type (0 = float32); sums are float32 either way.
+template <int DT, bool VEC>
 __global__ void __launch_bounds__(kInvThreads)
-inv_gather_kernel(int n, int c, int m, long long warps_total, const float* __restrict__ grad_out,
+inv_gather_kernel(int n, int c, int m, long long warps_total, const feat_t<DT>* __restrict__ grad_out,
                   const float* __restrict__ weight, const int* __restrict__ off, const int* __restrict__ entries,
                   float* __restrict__ grad_points, int* __restrict__ long_queue) {
     __shared__ int s_e[kInvThreads / 32][kInvSortCap];
@@ -590,7 +667,7 @@ inv_gather_kernel(int n, int c, int m, long long warps_total, const float* __res
         if (lane == 0) long_queue[1 + atomicAdd(long_queue, 1)] = (int)gw;  // the order of the queue does not matter
         return;
     }
-    const float* __restrict__ go = grad_out + (size_t)cloud * n * c;
+    const feat_t<DT>* __restrict__ go = grad_out + (size_t)cloud * n * c;
     const float* __restrict__ wt = weight + (size_t)cloud * n3;
     float* __restrict__ gp = grad_points + ((size_t)cloud * m + i) * c;
     {
@@ -616,15 +693,15 @@ inv_gather_kernel(int n, int c, int m, long long warps_total, const float* __res
         for (int sidx = 0; sidx < len; ++sidx) {
             const int e = s_e[wib][sidx];
             const float w = __ldg(wt + e);
-            const float* __restrict__ src = go + (size_t)(e / 3) * c + l;
+            const feat_t<DT>* __restrict__ src = go + (size_t)(e / 3) * c + l;
             if (VEC) {
-                const float4 g = __ldg(reinterpret_cast<const float4*>(src));
+                const float4 g = ld_grad4<DT>(src);
                 a0 = __fadd_rn(a0, __fmul_rn(g.x, w));
                 a1 = __fadd_rn(a1, __fmul_rn(g.y, w));
                 a2 = __fadd_rn(a2, __fmul_rn(g.z, w));
                 a3 = __fadd_rn(a3, __fmul_rn(g.w, w));
             } else {
-                a0 = __fadd_rn(a0, __fmul_rn(__ldg(src), w));
+                a0 = __fadd_rn(a0, __fmul_rn(ld_grad1<DT>(src), w));
             }
         }
         if (VEC) *reinterpret_cast<float4*>(gp + l) = make_float4(a0, a1, a2, a3);
@@ -637,9 +714,9 @@ inv_gather_kernel(int n, int c, int m, long long warps_total, const float* __res
 // (coalesced index loads + ballot), adds the entries that point at i in that order, and the 8 partial sums are
 // combined in piece order — a fixed association, hence deterministic (it differs from one long sequential sum
 // only in rounding; short lists, the normal case, are bit-identical to the reference's loop).
-template <bool VEC>
+template <int DT, bool VEC>
 __global__ void __launch_bounds__(kInvThreads)
-inv_long_kernel(int n, int c, int m, const float* __restrict__ grad_out, const int* __restrict__ idx,
+inv_long_kernel(int n, int c, int m, const feat_t<DT>* __restrict__ grad_out, const int* __restrict__ idx,
                 const float* __restrict__ weight, const int* __restrict__ long_queue, float* __restrict__ grad_points) {
     constexpr int NW = kInvThreads / 32;
     constexpr int W = VEC ? 4 : 1;
@@ -652,7 +729,7 @@ inv_long_kernel(int n, int c, int m, const float* __restrict__ grad_out, const i
         const long long gw = long_queue[1 + q];
         const long long cloud = gw / m;
         const int i = (int)(gw - cloud * m);
-        const float* __restrict__ go = grad_out + (size_t)cloud * n * c;
+        const feat_t<DT>* __restrict__ go = grad_out + (size_t)cloud * n * c;
         const float* __restrict__ wt = weight + (size_t)cloud * n3;
         const int* __restrict__ cidx = idx + cloud * n3;
         float* __restrict__ gp = grad_points + ((size_t)cloud * m + i) * c;
@@ -682,9 +759,9 @@ inv_long_kernel(int n, int c, int m, const float* __restrict__ grad_out, const i
                         w[u] = 0.f;
                         if (ee[u] >= 0 && act) {
                             w[u] = __ldg(wt + ee[u]);
-                            const float* __restrict__ src = go + (size_t)(ee[u] / 3) * c + l;
-                            if (VEC) g[u] = __ldg(reinterpret_cast<const float4*>(src));
-                            else g[u].x = __ldg(src);
+                            const feat_t<DT>* __restrict__ src = go + (size_t)(ee[u] / 3) * c + l;
+                            if (VEC) g[u] = ld_grad4<DT>(src);
+                            else g[u].x = ld_grad1<DT>(src);
                         }
                     }
 #pragma unroll
@@ -730,6 +807,182 @@ static unsigned it_grid(unsigned long long work_items, unsigned per_block) {
 }
 
 static bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+// ---- 16-bit features (pn2_*_h) -------------------------------------------------------------------
+// three_interpolate: one thread per 8 output values (16-byte loads of each of the three rows) when c % 8 == 0 and the
+// bases are 16-byte aligned, else one per value.  Values widened exactly, interp3 in float32, one rounding.
+template <typename IndexT, int DT>
+__global__ void __launch_bounds__(kItThreads)
+three_interp_h_vec8_kernel(int m, int c8, IndexT rows_per_cloud, IndexT total_vec, const uint4* __restrict__ points,
+                           const int* __restrict__ idx, const float* __restrict__ weight, uint4* __restrict__ out) {
+    const IndexT stride = (IndexT)gridDim.x * kItThreads;
+    for (IndexT v = (IndexT)blockIdx.x * kItThreads + threadIdx.x; v < total_vec; v += stride) {
+        const IndexT row = v / (IndexT)c8;
+        const int l = (int)(v - row * (IndexT)c8);
+        const IndexT cloud = row / rows_per_cloud;
+        const int i1 = __ldg(idx + (size_t)row * 3 + 0), i2 = __ldg(idx + (size_t)row * 3 + 1), i3 = __ldg(idx + (size_t)row * 3 + 2);
+        const float w1 = __ldg(weight + (size_t)row * 3 + 0), w2 = __ldg(weight + (size_t)row * 3 + 1),
+                    w3 = __ldg(weight + (size_t)row * 3 + 2);
+        const uint4* pb = points + (size_t)cloud * m * c8 + l;
+        const uint4 a = __ldg(pb + (size_t)i1 * c8), b = __ldg(pb + (size_t)i2 * c8), c = __ldg(pb + (size_t)i3 * c8);
+        __stcs(out + v, interp3_h8<DT>(a, b, c, w1, w2, w3));
+    }
+}
+
+template <typename IndexT, int DT>
+__global__ void __launch_bounds__(kItThreads)
+three_interp_h_scalar_kernel(int m, int c, IndexT rows_per_cloud, IndexT total, const unsigned short* __restrict__ points,
+                             const int* __restrict__ idx, const float* __restrict__ weight, unsigned short* __restrict__ out) {
+    const IndexT stride = (IndexT)gridDim.x * kItThreads;
+    for (IndexT e = (IndexT)blockIdx.x * kItThreads + threadIdx.x; e < total; e += stride) {
+        const IndexT row = e / (IndexT)c;
+        const int l = (int)(e - row * (IndexT)c);
+        const IndexT cloud = row / rows_per_cloud;
+        const int* ii = idx + (size_t)row * 3;
+        const float* w = weight + (size_t)row * 3;
+        const unsigned short* pb = points + (size_t)cloud * m * c + l;
+        out[e] = f_to_h<DT>(interp3(h_to_f<DT>(__ldg(pb + (size_t)__ldg(ii + 0) * c)), h_to_f<DT>(__ldg(pb + (size_t)__ldg(ii + 1) * c)),
+                                    h_to_f<DT>(__ldg(pb + (size_t)__ldg(ii + 2) * c)), __ldg(w + 0), __ldg(w + 1), __ldg(w + 2)));
+    }
+}
+
+template <int DT>
+static int three_interp_h(int b, int m, int c, int n, const unsigned short* points, const int* idx, const float* weight,
+                          unsigned short* out, cudaStream_t st) {
+    const unsigned long long total = (unsigned long long)b * n * c;
+    if (c % 8 == 0 && al16(points) && al16(out)) {
+        const unsigned long long tv = total / 8;
+        const unsigned grid = it_grid(tv, kItThreads);
+        const uint4* p8 = reinterpret_cast<const uint4*>(points);
+        uint4* o8 = reinterpret_cast<uint4*>(out);
+        if (tv < (1ull << 31))
+            three_interp_h_vec8_kernel<unsigned, DT><<<grid, kItThreads, 0, st>>>(m, c / 8, (unsigned)n, (unsigned)tv, p8, idx, weight, o8);
+        else
+            three_interp_h_vec8_kernel<unsigned long long, DT><<<grid, kItThreads, 0, st>>>(m, c / 8, (unsigned long long)n, tv, p8, idx, weight, o8);
+    } else {
+        const unsigned grid = it_grid(total, kItThreads);
+        if (total < (1ull << 31))
+            three_interp_h_scalar_kernel<unsigned, DT><<<grid, kItThreads, 0, st>>>(m, c, (unsigned)n, (unsigned)total, points, idx, weight, out);
+        else
+            three_interp_h_scalar_kernel<unsigned long long, DT><<<grid, kItThreads, 0, st>>>(m, c, (unsigned long long)n, total, points, idx, weight, out);
+    }
+    return finish_launch();
+}
+
+// grad_points[b, idx[b,j,t], l] += grad_out[b,j,l] * weight[b,j,t] with a 16-bit grad_out, float atomics into float32.
+// VEC: 4 channels per thread (8-byte loads, red.global.add.v4.f32), c % 4 == 0.
+template <typename IndexT, int DT, bool VEC>
+__global__ void __launch_bounds__(kItThreads)
+three_interp_grad_h_kernel(int m, int c, IndexT rows_per_cloud, IndexT total, const unsigned short* __restrict__ grad_out,
+                           const int* __restrict__ idx, const float* __restrict__ weight, float* __restrict__ grad_points) {
+    constexpr int W = VEC ? 4 : 1;
+    const int cw = c / W;
+    const IndexT stride = (IndexT)gridDim.x * kItThreads;
+    for (IndexT e = (IndexT)blockIdx.x * kItThreads + threadIdx.x; e < total; e += stride) {
+        const IndexT row = e / (IndexT)cw;
+        const int l = (int)(e - row * (IndexT)cw) * W;
+        const IndexT cloud = row / rows_per_cloud;
+        float4 g;
+        if (VEC) {
+            const uint2 u = __ldcs(reinterpret_cast<const uint2*>(grad_out) + e);
+            const float2 lo = h2_to_f2<DT>(u.x), hi = h2_to_f2<DT>(u.y);
+            g = make_float4(lo.x, lo.y, hi.x, hi.y);
+        } else {
+            g.x = h_to_f<DT>(__ldcs(grad_out + e));
+        }
+        float* gb = grad_points + (size_t)cloud * m * c + l;
+#pragma unroll
+        for (int t = 0; t < 3; ++t) {
+            const int i = __ldg(idx + (size_t)row * 3 + t);
+            const float w = __ldg(weight + (size_t)row * 3 + t);
+            if (VEC)
+                atomicAdd(reinterpret_cast<float4*>(gb + (size_t)i * c),
+                          make_float4(__fmul_rn(g.x, w), __fmul_rn(g.y, w), __fmul_rn(g.z, w), __fmul_rn(g.w, w)));
+            else
+                atomicAdd(gb + (size_t)i * c, __fmul_rn(g.x, w));
+        }
+    }
+}
+
+template <int DT>
+static int three_interp_grad_h(int b, int n, int c, int m, const unsigned short* grad_out, const int* idx, const float* weight,
+                               float* grad_points, cudaStream_t st) {
+    const unsigned long long total = (unsigned long long)b * n * c;
+    if (c % 4 == 0 && (reinterpret_cast<uintptr_t>(grad_out) & 7u) == 0 && al16(grad_points)) {
+        const unsigned long long tv = total / 4;
+        const unsigned grid = it_grid(tv, kItThreads);
+        if (tv < (1ull << 31))
+            three_interp_grad_h_kernel<unsigned, DT, true><<<grid, kItThreads, 0, st>>>(m, c, (unsigned)n, (unsigned)tv, grad_out, idx, weight, grad_points);
+        else
+            three_interp_grad_h_kernel<unsigned long long, DT, true><<<grid, kItThreads, 0, st>>>(m, c, (unsigned long long)n, tv, grad_out, idx, weight, grad_points);
+    } else {
+        const unsigned grid = it_grid(total, kItThreads);
+        if (total < (1ull << 31))
+            three_interp_grad_h_kernel<unsigned, DT, false><<<grid, kItThreads, 0, st>>>(m, c, (unsigned)n, (unsigned)total, grad_out, idx, weight, grad_points);
+        else
+            three_interp_grad_h_kernel<unsigned long long, DT, false><<<grid, kItThreads, 0, st>>>(m, c, (unsigned long long)n, total, grad_out, idx, weight, grad_points);
+    }
+    return finish_launch();
+}
+
+// pn2_three_interpolate_grad_det for a float32 (DT = 0) or 16-bit grad_out: the inverse index does not depend on it
+template <int DT>
+static int three_interp_grad_det(int b, int n, int c, int m, const feat_t<DT>* grad_out, const int* idx, const float* weight,
+                                 float* grad_points, void* workspace, size_t workspace_bytes, void* stream) {
+    if (b < 0 || m <= 0 || c < 0 || n < 0) return (int)cudaErrorInvalidValue;
+    if ((unsigned long long)b * m * c == 0) return 0;
+    if (!grad_points) return (int)cudaErrorInvalidValue;
+    cudaStream_t st = as_stream(stream);
+    if (n == 0) return (int)cudaMemsetAsync(grad_points, 0, sizeof(float) * (size_t)b * m * c, st);
+    if (!grad_out || !idx || !weight || !workspace) return (int)cudaErrorInvalidValue;
+    if (workspace_bytes < ::pn2_three_interpolate_grad_det_workspace_bytes(b, n, m) || (long long)n * 3 > 0x7fffffffLL)
+        return (int)cudaErrorInvalidValue;
+    int* off = static_cast<int*>(workspace);
+    int* cur = off + (size_t)b * (m + 1);
+    int* entries = cur + (size_t)b * m;
+    int* long_queue = entries + (size_t)b * 3 * (size_t)n;  // [0] = count, then (cloud * m + i) of every list > kInvSortCap
+    int launches = 2;
+    if (m <= kInvBuildMaxM) {
+        static std::atomic<unsigned long long> attr_done{0ull};
+        int dev = 0;
+        cudaError_t e = cudaGetDevice(&dev);
+        if (e != cudaSuccess) return (int)e;
+        if (dev >= 64 || !(attr_done.load(std::memory_order_acquire) & (1ull << dev))) {
+            e = cudaFuncSetAttribute(inv_build_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(int) * (kInvBuildMaxM + 1));
+            if (e != cudaSuccess) return (int)e;
+            if (dev < 64) attr_done.fetch_or(1ull << dev, std::memory_order_release);
+        }
+        inv_build_kernel<<<b, 1024, sizeof(int) * (size_t)(m + 1), st>>>(3 * n, m, idx, off, entries, long_queue);
+        launches += 1;
+    } else {
+        cudaError_t e = cudaMemsetAsync(off, 0, sizeof(int) * (size_t)b * (m + 1), st);
+        if (e == cudaSuccess) e = cudaMemsetAsync(long_queue, 0, sizeof(int), st);
+        if (e != cudaSuccess) return (int)e;
+        const long long total = (long long)b * n * 3;
+        const unsigned g1 = it_grid((unsigned long long)total, kInvThreads);
+        inv_count_kernel<<<g1, kInvThreads, 0, st>>>(3 * n, m, total, idx, off);
+        inv_scan_kernel<<<b, 1024, 0, st>>>(m, off, cur);
+        inv_fill_kernel<<<g1, kInvThreads, 0, st>>>(3 * n, m, total, idx, cur, entries);
+        launches += 3;
+    }
+    const long long warps = (long long)b * m;
+    const unsigned long long blocks = ((unsigned long long)warps * 32 + kInvThreads - 1) / kInvThreads;
+    if (blocks > 0x7fffffffull) return (int)cudaErrorInvalidValue;
+    // long lists: a fixed grid walks the queue (usually empty: the CTAs read one word and leave)
+    const unsigned long_grid = 148u * 2u;
+    // VEC: 4 channels per lane (16-byte float32 / 8-byte 16-bit loads)
+    const uintptr_t galign = DT == 0 ? 15u : 7u;
+    if (c % 4 == 0 && (reinterpret_cast<uintptr_t>(grad_out) & galign) == 0 && al16(grad_points)) {
+        inv_gather_kernel<DT, true><<<(unsigned)blocks, kInvThreads, 0, st>>>(n, c, m, warps, grad_out, weight, off, entries, grad_points, long_queue);
+        inv_long_kernel<DT, true><<<long_grid, kInvThreads, 0, st>>>(n, c, m, grad_out, idx, weight, long_queue, grad_points);
+    } else {
+        inv_gather_kernel<DT, false><<<(unsigned)blocks, kInvThreads, 0, st>>>(n, c, m, warps, grad_out, weight, off, entries, grad_points, long_queue);
+        inv_long_kernel<DT, false><<<long_grid, kInvThreads, 0, st>>>(n, c, m, grad_out, idx, weight, long_queue, grad_points);
+    }
+    count_launch(launches - 1);
+    return finish_launch();
+}
+
 
 }  // namespace pn2
 
@@ -803,7 +1056,7 @@ int pn2_three_nn_interpolate(int b, int n, int m, int c, const float* xyz1, cons
     if (b == 0 || n == 0) return 0;
     if (!xyz1 || !xyz2 || (c > 0 && (!points2 || !out))) return (int)cudaErrorInvalidValue;
     if (b > 65535) return (int)cudaErrorInvalidValue;
-    return fp_front_dispatch(b, n, m, c, 0, xyz1, xyz2, nullptr, points2, c > 0 ? out : nullptr, dist, idx, weight, as_stream(stream));
+    return fp_front_dispatch<0>(b, n, m, c, 0, xyz1, xyz2, nullptr, points2, c > 0 ? out : nullptr, dist, idx, weight, as_stream(stream));
 }
 
 int pn2_fp_interpolate_concat(int b, int n, int m, int c2, int c1, const float* xyz1, const float* xyz2, const float* points1,
@@ -813,7 +1066,7 @@ int pn2_fp_interpolate_concat(int b, int n, int m, int c2, int c1, const float* 
     if (b == 0 || n == 0) return 0;
     if (!xyz1 || !xyz2 || !points2 || !out || (c1 > 0 && !points1)) return (int)cudaErrorInvalidValue;
     if (b > 65535) return (int)cudaErrorInvalidValue;
-    return fp_front_dispatch(b, n, m, c2, c1, xyz1, xyz2, c1 > 0 ? points1 : nullptr, points2, out, nullptr, nullptr, nullptr,
+    return fp_front_dispatch<0>(b, n, m, c2, c1, xyz1, xyz2, c1 > 0 ? points1 : nullptr, points2, out, nullptr, nullptr, nullptr,
                              as_stream(stream));
 }
 
@@ -826,57 +1079,75 @@ size_t pn2_three_interpolate_grad_det_workspace_bytes(int b, int n, int m) {
 
 int pn2_three_interpolate_grad_det(int b, int n, int c, int m, const float* grad_out, const int* idx, const float* weight,
                                    float* grad_points, void* workspace, size_t workspace_bytes, void* stream) {
+    return pn2::three_interp_grad_det<0>(b, n, c, m, grad_out, idx, weight, grad_points, workspace, workspace_bytes, stream);
+}
+
+int pn2_three_interpolate_h(int dtype, int b, int m, int c, int n, const void* points, const int* idx, const float* weight,
+                            void* out, void* stream) {
     using namespace pn2;
+    if (!valid_half_dtype(dtype)) return (int)cudaErrorInvalidValue;
     if (b < 0 || m <= 0 || c < 0 || n < 0) return (int)cudaErrorInvalidValue;
-    if ((unsigned long long)b * m * c == 0) return 0;
-    if (!grad_points) return (int)cudaErrorInvalidValue;
-    cudaStream_t st = as_stream(stream);
-    if (n == 0) return (int)cudaMemsetAsync(grad_points, 0, sizeof(float) * (size_t)b * m * c, st);
-    if (!grad_out || !idx || !weight || !workspace) return (int)cudaErrorInvalidValue;
-    if (workspace_bytes < pn2_three_interpolate_grad_det_workspace_bytes(b, n, m) || (long long)n * 3 > 0x7fffffffLL)
-        return (int)cudaErrorInvalidValue;
-    int* off = static_cast<int*>(workspace);
-    int* cur = off + (size_t)b * (m + 1);
-    int* entries = cur + (size_t)b * m;
-    int* long_queue = entries + (size_t)b * 3 * (size_t)n;  // [0] = count, then (cloud * m + i) of every list > kInvSortCap
-    int launches = 2;
-    if (m <= kInvBuildMaxM) {
-        static std::atomic<unsigned long long> attr_done{0ull};
-        int dev = 0;
-        cudaError_t e = cudaGetDevice(&dev);
-        if (e != cudaSuccess) return (int)e;
-        if (dev >= 64 || !(attr_done.load(std::memory_order_acquire) & (1ull << dev))) {
-            e = cudaFuncSetAttribute(inv_build_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(int) * (kInvBuildMaxM + 1));
-            if (e != cudaSuccess) return (int)e;
-            if (dev < 64) attr_done.fetch_or(1ull << dev, std::memory_order_release);
-        }
-        inv_build_kernel<<<b, 1024, sizeof(int) * (size_t)(m + 1), st>>>(3 * n, m, idx, off, entries, long_queue);
-        launches += 1;
-    } else {
-        cudaError_t e = cudaMemsetAsync(off, 0, sizeof(int) * (size_t)b * (m + 1), st);
-        if (e == cudaSuccess) e = cudaMemsetAsync(long_queue, 0, sizeof(int), st);
-        if (e != cudaSuccess) return (int)e;
-        const long long total = (long long)b * n * 3;
-        const unsigned g1 = it_grid((unsigned long long)total, kInvThreads);
-        inv_count_kernel<<<g1, kInvThreads, 0, st>>>(3 * n, m, total, idx, off);
-        inv_scan_kernel<<<b, 1024, 0, st>>>(m, off, cur);
-        inv_fill_kernel<<<g1, kInvThreads, 0, st>>>(3 * n, m, total, idx, cur, entries);
-        launches += 3;
-    }
-    const long long warps = (long long)b * m;
-    const unsigned long long blocks = ((unsigned long long)warps * 32 + kInvThreads - 1) / kInvThreads;
-    if (blocks > 0x7fffffffull) return (int)cudaErrorInvalidValue;
-    // long lists: a fixed grid walks the queue (usually empty: the CTAs read one word and leave)
-    const unsigned long_grid = 148u * 2u;
-    if (c % 4 == 0 && al16(grad_out) && al16(grad_points)) {
-        inv_gather_kernel<true><<<(unsigned)blocks, kInvThreads, 0, st>>>(n, c, m, warps, grad_out, weight, off, entries, grad_points, long_queue);
-        inv_long_kernel<true><<<long_grid, kInvThreads, 0, st>>>(n, c, m, grad_out, idx, weight, long_queue, grad_points);
-    } else {
-        inv_gather_kernel<false><<<(unsigned)blocks, kInvThreads, 0, st>>>(n, c, m, warps, grad_out, weight, off, entries, grad_points, long_queue);
-        inv_long_kernel<false><<<long_grid, kInvThreads, 0, st>>>(n, c, m, grad_out, idx, weight, long_queue, grad_points);
-    }
-    count_launch(launches - 1);
-    return finish_launch();
+    if ((unsigned long long)b * n * c == 0) return 0;
+    if (!points || !idx || !weight || !out) return (int)cudaErrorInvalidValue;
+    const unsigned short* p = static_cast<const unsigned short*>(points);
+    unsigned short* o = static_cast<unsigned short*>(out);
+    if (dtype == PN2_DTYPE_BF16) return three_interp_h<PN2_DTYPE_BF16>(b, m, c, n, p, idx, weight, o, as_stream(stream));
+    return three_interp_h<PN2_DTYPE_F16>(b, m, c, n, p, idx, weight, o, as_stream(stream));
+}
+
+int pn2_three_interpolate_grad_h(int dtype, int b, int n, int c, int m, const void* grad_out, const int* idx,
+                                 const float* weight, float* grad_points, void* stream) {
+    using namespace pn2;
+    if (!valid_half_dtype(dtype)) return (int)cudaErrorInvalidValue;
+    if (b < 0 || m <= 0 || c < 0 || n < 0) return (int)cudaErrorInvalidValue;
+    if ((unsigned long long)b * n * c == 0) return 0;
+    if (!grad_out || !idx || !weight || !grad_points) return (int)cudaErrorInvalidValue;
+    const unsigned short* g = static_cast<const unsigned short*>(grad_out);
+    if (dtype == PN2_DTYPE_BF16) return three_interp_grad_h<PN2_DTYPE_BF16>(b, n, c, m, g, idx, weight, grad_points, as_stream(stream));
+    return three_interp_grad_h<PN2_DTYPE_F16>(b, n, c, m, g, idx, weight, grad_points, as_stream(stream));
+}
+
+int pn2_three_interpolate_grad_det_h(int dtype, int b, int n, int c, int m, const void* grad_out, const int* idx,
+                                     const float* weight, float* grad_points, void* workspace, size_t workspace_bytes,
+                                     void* stream) {
+    using namespace pn2;
+    const unsigned short* g = static_cast<const unsigned short*>(grad_out);
+    if (dtype == PN2_DTYPE_BF16)
+        return three_interp_grad_det<PN2_DTYPE_BF16>(b, n, c, m, g, idx, weight, grad_points, workspace, workspace_bytes, stream);
+    if (dtype == PN2_DTYPE_F16)
+        return three_interp_grad_det<PN2_DTYPE_F16>(b, n, c, m, g, idx, weight, grad_points, workspace, workspace_bytes, stream);
+    return (int)cudaErrorInvalidValue;
+}
+
+int pn2_three_nn_interpolate_h(int dtype, int b, int n, int m, int c, const float* xyz1, const float* xyz2, const void* points2,
+                               void* out, float* dist, int* idx, float* weight, void* stream) {
+    using namespace pn2;
+    if (!valid_half_dtype(dtype)) return (int)cudaErrorInvalidValue;
+    if (b < 0 || n < 0 || m <= 0 || c < 0) return (int)cudaErrorInvalidValue;
+    if (b == 0 || n == 0) return 0;
+    if (!xyz1 || !xyz2 || (c > 0 && (!points2 || !out))) return (int)cudaErrorInvalidValue;
+    if (b > 65535) return (int)cudaErrorInvalidValue;
+    const unsigned short* p2 = static_cast<const unsigned short*>(points2);
+    unsigned short* o = c > 0 ? static_cast<unsigned short*>(out) : nullptr;
+    if (dtype == PN2_DTYPE_BF16)
+        return fp_front_dispatch<PN2_DTYPE_BF16>(b, n, m, c, 0, xyz1, xyz2, nullptr, p2, o, dist, idx, weight, as_stream(stream));
+    return fp_front_dispatch<PN2_DTYPE_F16>(b, n, m, c, 0, xyz1, xyz2, nullptr, p2, o, dist, idx, weight, as_stream(stream));
+}
+
+int pn2_fp_interpolate_concat_h(int dtype, int b, int n, int m, int c2, int c1, const float* xyz1, const float* xyz2,
+                                const void* points1, const void* points2, void* out, void* stream) {
+    using namespace pn2;
+    if (!valid_half_dtype(dtype)) return (int)cudaErrorInvalidValue;
+    if (b < 0 || n < 0 || m <= 0 || c2 <= 0 || c1 < 0) return (int)cudaErrorInvalidValue;
+    if (b == 0 || n == 0) return 0;
+    if (!xyz1 || !xyz2 || !points2 || !out || (c1 > 0 && !points1)) return (int)cudaErrorInvalidValue;
+    if (b > 65535) return (int)cudaErrorInvalidValue;
+    const unsigned short* p1 = c1 > 0 ? static_cast<const unsigned short*>(points1) : nullptr;
+    const unsigned short* p2 = static_cast<const unsigned short*>(points2);
+    unsigned short* o = static_cast<unsigned short*>(out);
+    if (dtype == PN2_DTYPE_BF16)
+        return fp_front_dispatch<PN2_DTYPE_BF16>(b, n, m, c2, c1, xyz1, xyz2, p1, p2, o, nullptr, nullptr, nullptr, as_stream(stream));
+    return fp_front_dispatch<PN2_DTYPE_F16>(b, n, m, c2, c1, xyz1, xyz2, p1, p2, o, nullptr, nullptr, nullptr, as_stream(stream));
 }
 
 }  // extern "C"

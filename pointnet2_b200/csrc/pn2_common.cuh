@@ -1,7 +1,11 @@
 // pn2_common.cuh — shared device/host helpers for libpn2_b200 (sm_100a only).
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+
+#include <type_traits>
 
 #include "pn2_api.h"
 
@@ -108,6 +112,35 @@ int launch_ball_query_brute(int b, int n, int m, float thr, int nsample, const f
 int fps_dispatch(int b, int n, int m, const float* inp, float* temp, int* out, float* new_xyz, int sentinel, cudaStream_t st);
 bool fps_single_cta(int b, int n);
 size_t fps_scratch_bytes(int b, int n);
+
+// ---- 16-bit features (the pn2_*_h entry points) -------------------------------------------------
+// DT = 0 for float32, PN2_DTYPE_BF16 or PN2_DTYPE_F16; 16-bit values travel as their bit patterns.
+template <int DT>
+using feat_t = std::conditional_t<DT == 0, float, unsigned short>;
+
+inline bool valid_half_dtype(int dt) { return dt == PN2_DTYPE_BF16 || dt == PN2_DTYPE_F16; }
+
+// exact widening
+template <int DT>
+__device__ __forceinline__ float h_to_f(unsigned short u) {
+    if (DT == PN2_DTYPE_BF16) return __uint_as_float((unsigned)u << 16);
+    return __half2float(__ushort_as_half(u));
+}
+// one rounding, to nearest-even
+template <int DT>
+__device__ __forceinline__ unsigned short f_to_h(float f) {
+    if (DT == PN2_DTYPE_BF16) return __bfloat16_as_ushort(__float2bfloat16_rn(f));
+    return __half_as_ushort(__float2half_rn(f));
+}
+// a word of two 16-bit values: element 2i is the low half
+template <int DT>
+__device__ __forceinline__ float2 h2_to_f2(unsigned w) {
+    return make_float2(h_to_f<DT>((unsigned short)(w & 0xffffu)), h_to_f<DT>((unsigned short)(w >> 16)));
+}
+template <int DT>
+__device__ __forceinline__ unsigned f2_to_h2(float lo, float hi) {
+    return (unsigned)f_to_h<DT>(lo) | ((unsigned)f_to_h<DT>(hi) << 16);
+}
 
 // ---- streaming memory ops ---------------------------------------------------------------------
 __device__ __forceinline__ void st_stream_f4(float4* p, float4 v) { __stcs(p, v); }

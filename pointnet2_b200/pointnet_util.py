@@ -20,7 +20,7 @@ from typing import Callable, Optional, Sequence
 import torch
 
 from . import _lib, layers
-from ._tensor import on_device, ptr, require_cuda, same_device, stream_ptr
+from ._tensor import feature_dtype_code, on_device, ptr, require_cuda, same_device, stream_ptr
 from .tf_grouping import group_point, knn_point, query_ball_point
 from .tf_interpolate import fp_interpolate_concat, three_interpolate, three_nn, three_nn_interpolate
 from .sa_layer import sample_group, sample_group_msg
@@ -28,32 +28,38 @@ from .tf_sampling import farthest_point_sample, farthest_point_sample_and_gather
 
 
 class _GroupConcat(torch.autograd.Function):
-    """out = concat(xyz[idx]-new_xyz, points[idx]) in either channel order, plus grouped_xyz."""
+    """out = concat(xyz[idx]-new_xyz, points[idx]) in either channel order, plus grouped_xyz.  ``out`` has the dtype of
+    ``points`` (float32 without points; the centred xyz rounded once into it), ``grouped_xyz`` is float32."""
 
     @staticmethod
-    def forward(ctx, xyz, new_xyz, points, idx, xyz_first):
+    def forward(ctx, xyz, new_xyz, points, idx, xyz_first, dt):
         b, n, _ = xyz.shape
         _, m, s = idx.shape
         c = 0 if points is None else points.shape[2]
-        out = torch.empty((b, m, s, 3 + c), dtype=torch.float32, device=xyz.device)
+        dtype = torch.float32 if points is None else points.dtype
+        out = torch.empty((b, m, s, 3 + c), dtype=dtype, device=xyz.device)
         gxyz = torch.empty((b, m, s, 3), dtype=torch.float32, device=xyz.device)
         if out.numel():
+            lib = _lib.load()
             with on_device(xyz):
-                rc = _lib.load().pn2_group_concat(b, n, c, m, s, ptr(xyz), ptr(new_xyz), ptr(points), ptr(idx),
-                                                  1 if xyz_first else 0, ptr(out), ptr(gxyz), stream_ptr(xyz.device))
+                args = (b, n, c, m, s, ptr(xyz), ptr(new_xyz), ptr(points), ptr(idx), 1 if xyz_first else 0, ptr(out),
+                        ptr(gxyz), stream_ptr(xyz.device))
+                rc = lib.pn2_group_concat_h(dt, *args) if dt else lib.pn2_group_concat(*args)
             _lib.check(rc, "pn2_group_concat")
         ctx.save_for_backward(idx)
-        ctx.meta = (b, n, c, m, s, bool(xyz_first), points is not None)
+        ctx.meta = (b, n, c, m, s, bool(xyz_first), points is not None, dt, dtype)
         return out, gxyz
 
     @staticmethod
     def backward(ctx, g_out, g_gxyz):
         (idx,) = ctx.saved_tensors
-        b, n, c, m, s, xyz_first, has_points = ctx.meta
+        b, n, c, m, s, xyz_first, has_points, dt, dtype = ctx.meta
         lib = _lib.load()
         dev = g_out.device
         lo = 0 if xyz_first else c
         g_xyz_part = g_out[..., lo:lo + 3]
+        if dt:  # coordinates' gradient in float32, through the float32 kernel
+            g_xyz_part = g_xyz_part.float()
         if g_gxyz is not None:
             g_xyz_part = g_xyz_part + g_gxyz
         g_xyz_part = g_xyz_part.contiguous()
@@ -64,21 +70,30 @@ class _GroupConcat(torch.autograd.Function):
             _lib.check(lib.pn2_group_point_grad(b, n, 3, m, s, ptr(g_xyz_part), ptr(idx), ptr(g_xyz), st),
                        "pn2_group_point_grad")
             if has_points:
-                g_feat = (g_out[..., 3:] if xyz_first else g_out[..., :c]).contiguous()
+                g_feat = (g_out[..., 3:] if xyz_first else g_out[..., :c]).to(dtype).contiguous()
                 g_points = torch.zeros((b, n, c), dtype=torch.float32, device=dev)
-                _lib.check(lib.pn2_group_point_grad(b, n, c, m, s, ptr(g_feat), ptr(idx), ptr(g_points), st),
-                           "pn2_group_point_grad")
+                if dt:  # 16-bit grad_out, accumulated in float32, rounded once
+                    _lib.check(lib.pn2_group_point_grad_h(dt, b, n, c, m, s, ptr(g_feat), ptr(idx), ptr(g_points), st),
+                               "pn2_group_point_grad_h")
+                    g_points = g_points.to(dtype)
+                else:
+                    _lib.check(lib.pn2_group_point_grad(b, n, c, m, s, ptr(g_feat), ptr(idx), ptr(g_points), st),
+                               "pn2_group_point_grad")
         g_new_xyz = -g_xyz_part.sum(dim=2)
-        return g_xyz, g_new_xyz, g_points, None, None
+        return g_xyz, g_new_xyz, g_points, None, None, None
 
 
 def group_and_concat(xyz, new_xyz, points, idx, xyz_first: bool = True):
-    """Fused tail of sample_and_group: returns (new_points (b,m,s,3+c), grouped_xyz (b,m,s,3))."""
+    """Fused tail of sample_and_group: returns (new_points (b,m,s,3+c), grouped_xyz (b,m,s,3)).
+
+    ``points`` may be float32, bfloat16 or float16; new_points then has its dtype (features copied bit for bit, the
+    centred xyz computed in float32 and rounded once).  xyz, new_xyz and grouped_xyz are float32."""
+    dt = 0 if points is None else feature_dtype_code(points, "points")
     xyz = require_cuda(xyz, "xyz", torch.float32)
     new_xyz = require_cuda(new_xyz, "new_xyz", torch.float32)
     idx = require_cuda(idx, "idx", torch.int32)
     if points is not None:
-        points = require_cuda(points, "points", torch.float32)
+        points = require_cuda(points, "points", points.dtype)
         same_device(xyz, new_xyz, idx, points)
         if points.dim() != 3 or points.shape[:2] != xyz.shape[:2]:
             raise ValueError("points must be (batch_size, ndataset, channel) matching xyz")
@@ -86,7 +101,7 @@ def group_and_concat(xyz, new_xyz, points, idx, xyz_first: bool = True):
         same_device(xyz, new_xyz, idx)
     if idx.dim() != 3 or idx.shape[0] != xyz.shape[0] or new_xyz.shape[:2] != idx.shape[:2]:
         raise ValueError("idx must be (batch_size, npoint, nsample) matching new_xyz")
-    return _GroupConcat.apply(xyz, new_xyz, points, idx, xyz_first)
+    return _GroupConcat.apply(xyz, new_xyz, points, idx, xyz_first, dt)
 
 
 def sample_and_group(npoint, radius, nsample, xyz, points, knn=False, use_xyz=True, fused=True):
@@ -95,7 +110,8 @@ def sample_and_group(npoint, radius, nsample, xyz, points, knn=False, use_xyz=Tr
 
     Args:
         npoint, radius, nsample: centroids to sample, ball radius, neighbours kept per centroid.
-        xyz (b, n, 3) float32; points (b, n, c) float32 or None (then the grouped xyz are the features).
+        xyz (b, n, 3) float32; points (b, n, c) float32, bfloat16 or float16, or None (then the grouped xyz are
+        the features).  new_points has the dtype of points; grouped_xyz is float32.
         knn: k-nearest-neighbour grouping instead of the ball query; use_xyz: keep the centred xyz
         in front of the grouped features.
     Returns:
@@ -259,7 +275,9 @@ def pointnet_fp_module(xyz1, xyz2, points1, points2, mlp=None, is_training=None,
         Return: new_points (b,n1,mlp[-1]) (or (b,n1,c2+c1) when mlp is None)
     '''
     no_grad = not points2.requires_grad and (points1 is None or not points1.requires_grad)
-    if fused and no_grad and points2.shape[2] > 0:
+    # the fused kernel takes one feature dtype; mixed ones go through torch.cat, which promotes
+    one_dtype = points1 is None or points1.dtype == points2.dtype
+    if fused and no_grad and one_dtype and points2.shape[2] > 0:
         # one kernel: 3-NN, weights, interpolation and the concat of :219
         new_points1 = fp_interpolate_concat(xyz1, xyz2, points1, points2)
     else:

@@ -9,7 +9,7 @@ from __future__ import annotations
 import torch
 
 from . import _lib
-from ._tensor import on_device, ptr, require_cuda, same_device, stream_ptr
+from ._tensor import feature_dtype_code, on_device, ptr, require_cuda, same_device, stream_ptr
 
 
 def query_ball_point(radius: float, nsample: int, xyz1: torch.Tensor, xyz2: torch.Tensor):
@@ -85,17 +85,21 @@ def select_top_k(k: int, dist: torch.Tensor):
 
 class _GroupPoint(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, points, idx):
+    def forward(ctx, points, idx, dt):
         b, n, c = points.shape
         _, m, s = idx.shape
-        out = torch.empty((b, m, s, c), dtype=torch.float32, device=points.device)
+        out = torch.empty((b, m, s, c), dtype=points.dtype, device=points.device)
         if out.numel():
+            lib = _lib.load()
             with on_device(points):
-                rc = _lib.load().pn2_group_point(b, n, c, m, s, ptr(points), ptr(idx), ptr(out),
-                                                 stream_ptr(points.device))
+                if dt:
+                    rc = lib.pn2_group_point_h(dt, b, n, c, m, s, ptr(points), ptr(idx), ptr(out), stream_ptr(points.device))
+                else:
+                    rc = lib.pn2_group_point(b, n, c, m, s, ptr(points), ptr(idx), ptr(out), stream_ptr(points.device))
             _lib.check(rc, "pn2_group_point")
         ctx.save_for_backward(idx)
         ctx.shape = (b, n, c)
+        ctx.dt = (dt, points.dtype)
         return out
 
     @staticmethod
@@ -103,26 +107,35 @@ class _GroupPoint(torch.autograd.Function):
         (idx,) = ctx.saved_tensors
         b, n, c = ctx.shape
         _, m, s = idx.shape
-        grad_out = grad_out.contiguous()
-        # zero-filled by the caller, as GroupPointGradGpuOp does (tf_grouping.cpp:204)
+        dt, dtype = ctx.dt
+        grad_out = grad_out.to(dtype).contiguous()
+        # zero-filled by the caller, as GroupPointGradGpuOp does (tf_grouping.cpp:204); 16-bit gradients accumulate in
+        # float32 and are rounded once
         grad_points = torch.zeros((b, n, c), dtype=torch.float32, device=grad_out.device)
         if grad_out.numel():
+            lib = _lib.load()
             with on_device(grad_out):
-                rc = _lib.load().pn2_group_point_grad(b, n, c, m, s, ptr(grad_out), ptr(idx), ptr(grad_points),
-                                                      stream_ptr(grad_out.device))
+                if dt:
+                    rc = lib.pn2_group_point_grad_h(dt, b, n, c, m, s, ptr(grad_out), ptr(idx), ptr(grad_points),
+                                                    stream_ptr(grad_out.device))
+                else:
+                    rc = lib.pn2_group_point_grad(b, n, c, m, s, ptr(grad_out), ptr(idx), ptr(grad_points),
+                                                  stream_ptr(grad_out.device))
             _lib.check(rc, "pn2_group_point_grad")
-        return grad_points, None
+        return grad_points.to(dtype), None, None
 
 
 def group_point(points: torch.Tensor, idx: torch.Tensor) -> torch.Tensor:
     """Row gather: ``out[b, j, s, :] = points[b, idx[b, j, s], :]``.
 
-    Arguments: ``points`` float32 (B, N, C), the rows to pick from; ``idx`` int32 (B, M, S), row numbers into
-    ``points``.  Returns float32 (B, M, S, C).  Differentiable in ``points``.
+    Arguments: ``points`` float32, bfloat16 or float16 (B, N, C), the rows to pick from; ``idx`` int32 (B, M, S), row
+    numbers into ``points``.  Returns (B, M, S, C) of the dtype of ``points``, bit for bit.  Differentiable in
+    ``points``; a 16-bit gradient is accumulated in float32 and rounded once.
     Reference: tf_grouping.py:33-41 -> group_point_gpu (tf_grouping_g.cu:40-57); gradient
     tf_grouping.py:42-46 -> group_point_grad_gpu (:61-78).
     """
-    points = require_cuda(points, "points", torch.float32)
+    dt = feature_dtype_code(points, "points")
+    points = require_cuda(points, "points", points.dtype)
     idx = require_cuda(idx, "idx", torch.int32)
     same_device(points, idx)
     if points.dim() != 3:
@@ -131,7 +144,7 @@ def group_point(points: torch.Tensor, idx: torch.Tensor) -> torch.Tensor:
         raise ValueError(f"GroupPoint expects (batch_size, npoints, nsample) idx shape, got {tuple(idx.shape)}")
     if points.shape[1] <= 0 and idx.numel():
         raise ValueError("GroupPoint expects a non-empty points tensor")
-    return _GroupPoint.apply(points, idx)
+    return _GroupPoint.apply(points, idx, dt)
 
 
 def knn_point(k: int, xyz1: torch.Tensor, xyz2: torch.Tensor):

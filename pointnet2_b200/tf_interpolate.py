@@ -11,7 +11,7 @@ from __future__ import annotations
 import torch
 
 from . import _lib
-from ._tensor import on_device, ptr, require_cuda, same_device, stream_ptr
+from ._tensor import feature_dtype_code, on_device, ptr, require_cuda, same_device, stream_ptr
 
 
 def three_nn(xyz1: torch.Tensor, xyz2: torch.Tensor):
@@ -49,17 +49,23 @@ DETERMINISTIC_GRAD = True
 
 class _ThreeInterpolate(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, points, idx, weight):
+    def forward(ctx, points, idx, weight, dt):
         b, m, c = points.shape
         n = idx.shape[1]
-        out = torch.empty((b, n, c), dtype=torch.float32, device=points.device)
+        out = torch.empty((b, n, c), dtype=points.dtype, device=points.device)
         if out.numel():
+            lib = _lib.load()
             with on_device(points):
-                rc = _lib.load().pn2_three_interpolate(b, m, c, n, ptr(points), ptr(idx), ptr(weight), ptr(out),
-                                                       stream_ptr(points.device))
+                if dt:
+                    rc = lib.pn2_three_interpolate_h(dt, b, m, c, n, ptr(points), ptr(idx), ptr(weight), ptr(out),
+                                                     stream_ptr(points.device))
+                else:
+                    rc = lib.pn2_three_interpolate(b, m, c, n, ptr(points), ptr(idx), ptr(weight), ptr(out),
+                                                   stream_ptr(points.device))
             _lib.check(rc, "pn2_three_interpolate")
         ctx.save_for_backward(idx, weight)
         ctx.shape = (b, m, c)
+        ctx.dt = (dt, points.dtype)
         return out
 
     @staticmethod
@@ -67,9 +73,11 @@ class _ThreeInterpolate(torch.autograd.Function):
         idx, weight = ctx.saved_tensors
         b, m, c = ctx.shape
         n = idx.shape[1]
-        grad_out = grad_out.contiguous()
+        dt, dtype = ctx.dt
+        grad_out = grad_out.to(dtype).contiguous()
         lib = _lib.load()
         dev = grad_out.device
+        # 16-bit gradients: the _h entries read the 16-bit grad_out and accumulate in float32, rounded once here
         if DETERMINISTIC_GRAD and b * m * c:
             # inverse index + ordered accumulation: deterministic, bit-identical to threeinterpolate_grad_cpu
             # (tf_interpolate.cpp:131-153), and ~3x faster than the atomics at the sem-seg sizes
@@ -77,29 +85,39 @@ class _ThreeInterpolate(torch.autograd.Function):
             with on_device(grad_out):
                 wsb = int(lib.pn2_three_interpolate_grad_det_workspace_bytes(b, max(n, 1), m))
                 ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-                rc = lib.pn2_three_interpolate_grad_det(b, n, c, m, ptr(grad_out), ptr(idx), ptr(weight), ptr(grad_points),
-                                                        ptr(ws), wsb, stream_ptr(dev))
+                if dt:
+                    rc = lib.pn2_three_interpolate_grad_det_h(dt, b, n, c, m, ptr(grad_out), ptr(idx), ptr(weight),
+                                                              ptr(grad_points), ptr(ws), wsb, stream_ptr(dev))
+                else:
+                    rc = lib.pn2_three_interpolate_grad_det(b, n, c, m, ptr(grad_out), ptr(idx), ptr(weight), ptr(grad_points),
+                                                            ptr(ws), wsb, stream_ptr(dev))
             _lib.check(rc, "pn2_three_interpolate_grad_det")
-            return grad_points, None, None
+            return grad_points.to(dtype), None, None, None
         # zero-filled by the caller, as ThreeInterpolateGradOp does (tf_interpolate.cpp:258)
         grad_points = torch.zeros((b, m, c), dtype=torch.float32, device=dev)
         if grad_out.numel():
             with on_device(grad_out):
-                rc = lib.pn2_three_interpolate_grad(b, n, c, m, ptr(grad_out), ptr(idx), ptr(weight),
-                                                    ptr(grad_points), stream_ptr(dev))
+                if dt:
+                    rc = lib.pn2_three_interpolate_grad_h(dt, b, n, c, m, ptr(grad_out), ptr(idx), ptr(weight),
+                                                          ptr(grad_points), stream_ptr(dev))
+                else:
+                    rc = lib.pn2_three_interpolate_grad(b, n, c, m, ptr(grad_out), ptr(idx), ptr(weight),
+                                                        ptr(grad_points), stream_ptr(dev))
             _lib.check(rc, "pn2_three_interpolate_grad")
-        return grad_points, None, None
+        return grad_points.to(dtype), None, None, None
 
 
 def three_interpolate(points: torch.Tensor, idx: torch.Tensor, weight: torch.Tensor) -> torch.Tensor:
     """Weighted sum of three feature rows: ``out[b, i, :] = sum_t weight[b, i, t] * points[b, idx[b, i, t], :]``.
 
-    ``points`` float32 (B, m, c): features of the known points; ``idx`` int32 and ``weight`` float32, both (B, n, 3),
-    as produced from three_nn.  Returns float32 (B, n, c).  Differentiable in ``points``.
+    ``points`` float32, bfloat16 or float16 (B, m, c): features of the known points; ``idx`` int32 and ``weight``
+    float32, both (B, n, 3), as produced from three_nn.  Returns (B, n, c) of the dtype of ``points``: 16-bit features
+    are widened exactly, interpolated in float32 and rounded once.  Differentiable in ``points``.
     Reference: tf_interpolate.py:19-28 -> threeinterpolate_cpu (tf_interpolate.cpp:107-127);
     gradient :29-34 -> threeinterpolate_grad_cpu (:131-153).
     """
-    points = require_cuda(points, "points", torch.float32)
+    dt = feature_dtype_code(points, "points")
+    points = require_cuda(points, "points", points.dtype)
     idx = require_cuda(idx, "idx", torch.int32)
     weight = require_cuda(weight, "weight", torch.float32)
     same_device(points, idx, weight)
@@ -112,18 +130,20 @@ def three_interpolate(points: torch.Tensor, idx: torch.Tensor, weight: torch.Ten
         raise ValueError(f"ThreeInterpolate expects (b,n,3) weight shape, got {tuple(weight.shape)}")
     if points.shape[1] <= 0 and idx.numel():
         raise ValueError("ThreeInterpolate expects a non-empty points tensor")
-    return _ThreeInterpolate.apply(points, idx, weight.detach())
+    return _ThreeInterpolate.apply(points, idx, weight.detach(), dt)
 
 
 def three_nn_interpolate(xyz1: torch.Tensor, xyz2: torch.Tensor, points2: torch.Tensor, return_aux: bool = False):
     """Fused feature-propagation front end (utils/pointnet_util.py:211-216): three_nn, the
     inverse-distance weights (dist=max(dist,1e-10); w=(1/dist)/sum(1/dist)) and three_interpolate
     in one kernel; dist/idx/weight stay on chip unless ``return_aux``.  Forward only (use the
-    unfused ops when ``points2`` needs a gradient).
+    unfused ops when ``points2`` needs a gradient).  ``points2`` may be float32, bfloat16 or float16; ``out`` has its
+    dtype (interpolated in float32, rounded once), dist / weight are float32.
     Returns out (b,n,c) [, dist (b,n,3), idx (b,n,3), weight (b,n,3)]."""
+    dt = feature_dtype_code(points2, "points2")
     xyz1 = require_cuda(xyz1, "xyz1", torch.float32)
     xyz2 = require_cuda(xyz2, "xyz2", torch.float32)
-    points2 = require_cuda(points2, "points2", torch.float32)
+    points2 = require_cuda(points2, "points2", points2.dtype)
     same_device(xyz1, xyz2, points2)
     if xyz1.dim() != 3 or xyz1.shape[2] != 3 or xyz2.dim() != 3 or xyz2.shape[2] != 3 or xyz1.shape[0] != xyz2.shape[0]:
         raise ValueError("three_nn_interpolate expects (b,n,3) xyz1 and (b,m,3) xyz2")
@@ -135,14 +155,16 @@ def three_nn_interpolate(xyz1: torch.Tensor, xyz2: torch.Tensor, points2: torch.
     if m <= 0:
         raise ValueError("three_nn_interpolate expects at least one known point")
     dev = xyz1.device
-    out = torch.empty((b, n, c), dtype=torch.float32, device=dev)
+    out = torch.empty((b, n, c), dtype=points2.dtype, device=dev)
     dist = torch.empty((b, n, 3), dtype=torch.float32, device=dev) if return_aux else None
     idx = torch.empty((b, n, 3), dtype=torch.int32, device=dev) if return_aux else None
     weight = torch.empty((b, n, 3), dtype=torch.float32, device=dev) if return_aux else None
     if b * n:
+        lib = _lib.load()
         with on_device(xyz1):
-            rc = _lib.load().pn2_three_nn_interpolate(b, n, m, c, ptr(xyz1), ptr(xyz2), ptr(points2.detach()), ptr(out),
-                                                      ptr(dist), ptr(idx), ptr(weight), stream_ptr(dev))
+            args = (b, n, m, c, ptr(xyz1), ptr(xyz2), ptr(points2.detach()), ptr(out), ptr(dist), ptr(idx), ptr(weight),
+                    stream_ptr(dev))
+            rc = lib.pn2_three_nn_interpolate_h(dt, *args) if dt else lib.pn2_three_nn_interpolate(*args)
         _lib.check(rc, "pn2_three_nn_interpolate")
     if return_aux:
         return out, dist, idx, weight
@@ -152,10 +174,16 @@ def three_nn_interpolate(xyz1: torch.Tensor, xyz2: torch.Tensor, points2: torch.
 def fp_interpolate_concat(xyz1: torch.Tensor, xyz2: torch.Tensor, points1, points2: torch.Tensor) -> torch.Tensor:
     """The front end of pointnet_fp_module in one kernel (utils/pointnet_util.py:211-219): three_nn, the
     inverse-distance weights, three_interpolate AND the concat with ``points1``:
-    returns (b, n, c2 + c1) = [interpolated points2 | points1] (c1 = 0 when ``points1`` is None).  Forward only."""
+    returns (b, n, c2 + c1) = [interpolated points2 | points1] (c1 = 0 when ``points1`` is None).  Forward only.
+    ``points1`` and ``points2`` are float32, bfloat16 or float16, both of the same dtype, which the output has."""
+    dt = feature_dtype_code(points2, "points2")
+    if points1 is not None:
+        feature_dtype_code(points1, "points1")
+        if points1.dtype != points2.dtype:
+            raise TypeError(f"fp_interpolate_concat expects points1 and points2 of one dtype, got {points1.dtype} and {points2.dtype}")
     xyz1 = require_cuda(xyz1, "xyz1", torch.float32)
     xyz2 = require_cuda(xyz2, "xyz2", torch.float32)
-    points2 = require_cuda(points2, "points2", torch.float32)
+    points2 = require_cuda(points2, "points2", points2.dtype)
     same_device(xyz1, xyz2, points2)
     if xyz1.dim() != 3 or xyz1.shape[2] != 3 or xyz2.dim() != 3 or xyz2.shape[2] != 3 or xyz1.shape[0] != xyz2.shape[0]:
         raise ValueError("fp_interpolate_concat expects (b,n,3) xyz1 and (b,m,3) xyz2")
@@ -165,18 +193,19 @@ def fp_interpolate_concat(xyz1: torch.Tensor, xyz2: torch.Tensor, points1, point
     m, c2 = xyz2.shape[1], points2.shape[2]
     c1 = 0
     if points1 is not None:
-        points1 = require_cuda(points1, "points1", torch.float32)
+        points1 = require_cuda(points1, "points1", points1.dtype)
         same_device(xyz1, points1)
         if points1.dim() != 3 or points1.shape[:2] != xyz1.shape[:2]:
             raise ValueError("fp_interpolate_concat expects (b,n,c1) points1 matching xyz1")
         c1 = points1.shape[2]
     if m <= 0 or c2 <= 0:
         raise ValueError("fp_interpolate_concat expects at least one known point and one channel")
-    out = torch.empty((b, n, c2 + c1), dtype=torch.float32, device=xyz1.device)
+    out = torch.empty((b, n, c2 + c1), dtype=points2.dtype, device=xyz1.device)
     if b * n:
+        lib = _lib.load()
         with on_device(xyz1):
-            rc = _lib.load().pn2_fp_interpolate_concat(b, n, m, c2, c1, ptr(xyz1), ptr(xyz2),
-                                                       ptr(points1.detach()) if c1 else None, ptr(points2.detach()), ptr(out),
-                                                       stream_ptr(xyz1.device))
+            args = (b, n, m, c2, c1, ptr(xyz1), ptr(xyz2), ptr(points1.detach()) if c1 else None, ptr(points2.detach()),
+                    ptr(out), stream_ptr(xyz1.device))
+            rc = lib.pn2_fp_interpolate_concat_h(dt, *args) if dt else lib.pn2_fp_interpolate_concat(*args)
         _lib.check(rc, "pn2_fp_interpolate_concat")
     return out
